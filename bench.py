@@ -49,6 +49,32 @@ def peaks():
     return 6650.0, "fallback (B200_PROFILING.md 6.65 TB/s)"
 
 
+DUMP_SAMPLE = 1 << 22   # decoded bytes sampled for --dump-outputs (16 MB as float32)
+DUMP_SEED = 20261020
+
+
+def dump_sample_positions(out_size):
+    """The fixed, seeded byte positions of the decoded output that --dump-outputs keeps (all of it when it is small)."""
+    if out_size <= DUMP_SAMPLE:
+        return np.arange(out_size, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(out_size, DUMP_SAMPLE, replace=False))
+
+
+def dump_outputs(out_dir, rank, world, status, digest, sample):
+    """--dump-outputs: what the caller of the timed path received in its last timed step, as .npy files that two
+    builds can compare array for array.  float64 holds the int32 statuses and each 32-bit half of the uint64 digests
+    exactly; the decoded bytes are a seeded sample (dump_sample_positions), as float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    digest = np.asarray(digest, np.uint64)
+    arrays = {"status": np.asarray(status).astype(np.float64),
+              "digest_hi32": (digest >> np.uint64(32)).astype(np.float64),
+              "digest_lo32": (digest & np.uint64(0xFFFFFFFF)).astype(np.float64),
+              "output_sample": np.asarray(sample).astype(np.float32)}
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 def _emit(args, line):
     """The contract line: printed, unless this run is a nested measurement for the `configs` block of another line."""
     if getattr(args, "nested", False):
@@ -573,6 +599,11 @@ def run_ours(args):
     ms_total = ev0.elapsed_time(ev1)
     launches = ctx.launch_count - launches0
     assert (status == 0).all() and np.array_equal(digest, d.hash)
+    if getattr(args, "dump_outputs", None):
+        # taken before anything below writes d_out again
+        pos = torch.from_numpy(dump_sample_positions(out_size)).cuda()
+        dump = (status.copy(), digest.copy(), d_out[pos].cpu().numpy())
+        del pos
     # per-kernel durations for the roofline: in the timed steps the execute kernel overlaps the tail of the parse
     # kernel (separate streams), so its own duration is taken from two extra, untimed steps with the kernels back to back
     ctx.set_overlap(False)
@@ -717,6 +748,8 @@ def run_ours(args):
                                     "sample": f"first {n_s} entries of the same archive, {cores} threads, each entry into its own slot "
                                               f"of one output, best of 2 passes; single-thread: {v1:.3f} GB/s"}
         _emit(args, line)
+    if getattr(args, "dump_outputs", None):
+        dump_outputs(args.dump_outputs, rank, world, *dump)
     if world > 1 and not getattr(args, "nested", False):
         dist.destroy_process_group()
     ctx.close()
@@ -1015,7 +1048,12 @@ def main():
                     help="strong (default): ONE archive cut over the ranks; weak: one archive of --entries per rank")
     ap.add_argument("--no-configs", dest="configs", action="store_false",
                     help="skip the C3 / C4 / C5 block that the default single-GPU C2 line carries")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (per-entry status, XXH3-64 digest, a seeded "
+                         "sample of the decoded bytes) as DIR/<name>.npy; c2 and c4 only")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.workload not in ("c2", "c4")):
+        ap.error("--dump-outputs is implemented for --impl ours with --workload c2 or c4")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -1037,7 +1075,8 @@ def main():
                                    ("c4", run_ours, 8192, "zstd level-3 unpack + verify, 8192 entries x 128 KiB (1 GiB), frames written by the reference"),
                                    ("c5", run_c5, 16384, "one LZ4 entry of 16384 independent 64 KB blocks (1 GiB), block-sharded read")):
         sub = copy.copy(args)
-        sub.workload, sub.entries, sub.steps, sub.warmup, sub.no_cpu, sub.e2e_steps, sub.result = key, n_small, 5, 3, True, 2, None
+        sub.workload, sub.entries, sub.warmup, sub.no_cpu, sub.e2e_steps, sub.result = key, n_small, 3, True, 2, None
+        sub.dump_outputs = None
         try:
             fn(sub)
             r = sub.result

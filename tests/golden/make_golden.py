@@ -8,6 +8,7 @@ Outputs (all small, committed):
   xxh3_kat.json      — XXH3-64 seed-0 known answers: the upstream table
         (/root/reference/externals/xxHash/xxhsum.c:1246-1272, buffer generator :585-596) plus
         digests computed by the unmodified reference for more lengths
+  xxh3_random.json   — XXH3-64 of seeded random buffers (tests/test_oracle.py)
   lz4_cases.npz      — LZ4 frames written by the unmodified reference (LZ4F_compressFrame) for
         hand-picked inputs: linked / independent, stored blocks, checksums, content size, multi-block
   zstd_cases.npz     — zstd frames written by the unmodified reference (ZSTD_compress), several levels
@@ -57,6 +58,17 @@ def main():
     for n in extra:
         kat["reference_run"][str(n)] = f"{O.xxh3_ref(buf[:n]):016x}"
     json.dump(kat, open(os.path.join(HERE, "xxh3_kat.json"), "w"), indent=0)
+
+    # XXH3-64 of random buffers at the lengths tests/test_oracle.py::test_ref_agrees_on_xxh3_random_lengths draws.
+    # (The committed table was written with upstream xxHash 0.8.2, whose XXH3_64bits reproduces every digest of
+    # xxh3_kat.json; XXH3's output is frozen since 0.8.0, the version the reference pins.)
+    rng = np.random.default_rng(7)
+    rbuf = rng.integers(0, 256, 300000, dtype=np.uint8)
+    lengths = list(range(0, 300)) + [int(x) for x in rng.integers(300, 300000, 60)]
+    json.dump({"generator": "buf = numpy default_rng(7).integers(0, 256, 300000, uint8); lengths 0..299, then 60 of the same "
+                            "generator's integers(300, 300000)",
+               "xxh3_64": [[n, f"{O.xxh3_ref(rbuf[:n]):016x}"] for n in lengths]},
+              open(os.path.join(HERE, "xxh3_random.json"), "w"), indent=0)
 
     rng = np.random.default_rng(1234)
     inputs = {
