@@ -182,11 +182,18 @@ int zpb_pack_device(zpb_ctx *ctx, const uint8_t *d_in, uint64_t in_size, uint8_t
 int zpb_pack_host(zpb_ctx *ctx, const uint8_t *h_in, uint64_t in_size, uint8_t *h_out,
                   uint64_t out_size, const zpb_file *files, uint64_t n, uint64_t *comp_size,
                   uint64_t *digest, int32_t *status);
+/* LZ4 levels 3 and above (LZ4 HC in the reference, lz4frame.c:799-807).  0 (the default; env ZPB_LZ4HC=1 turns it on
+ * at zpb_create): such files get ZPB_ST_NOT_AVAILABLE.  1: they are compressed by the HC block compressor — hash chains
+ * searched up to a level-dependent depth and a cost-based parse per 64 KB block; levels above 12 act as 12.  The frames
+ * have the same layout as the fast path's (block-independent, 64 KB blocks).  Levels below 3, zstd and stored files are
+ * the same either way.  zpb_pack_host passes the setting on to its worker contexts on every call. */
+int zpb_set_lz4hc(zpb_ctx *ctx, int enabled);
 
 /* last kernel timing (CUDA events on the launching stream), for bench.py's roofline block */
 int zpb_last_kernel_ms(const zpb_ctx *ctx, float *unpack_ms, float *pack_ms);
-/* The last zpb_pack_device call by stage, summed over its rounds: the block compressor (lz4_pack_blocks_kernel, the
- * role of LZ4_compress_fast_extState under lz4frame.c:735-760) and the framing + XXH3 kernel (lz4_pack_kernel). */
+/* The last zpb_pack_device call by stage, summed over its rounds: the block compressors (lz4_pack_blocks_kernel, the
+ * role of LZ4_compress_fast_extState under lz4frame.c:735-760, and the HC kernels lz4hc_match_kernel + lz4hc_parse_kernel)
+ * and the framing + XXH3 kernel (lz4_pack_kernel). */
 int zpb_last_pack_stage_ms(const zpb_ctx *ctx, float *blocks_ms, float *frames_ms);
 
 /* per-stage device time of the last unpack (ms): scan, parse, exec, general-fallback.  With the overlap on (the

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """Developer benchmark for BASELINE config C3: LZ4 pack of the zpk-synth-v1 corpus, device-resident.
-Prints one JSON line: uncompressed GB/s, ratio vs the reference algorithm at level 0, kernel ms."""
+Prints one JSON line per class: uncompressed GB/s, ratio vs the reference algorithm at level 0, kernel ms; with
+--level N (LZ4 HC from 3 on) also the block / framing stage ms and the GPU's level-0 ratio on the same data."""
 import argparse
 import json
 import os
@@ -32,12 +33,22 @@ def main():
     ap.add_argument("--classes", default="-1")
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--method", type=int, default=2, help="2 = LZ4 (default), 1 = zstd")
+    ap.add_argument("--level", type=int, default=0, help="LZ4 level; >= 3 turns the context's HC switch on (zpb_set_lz4hc)")
     a = ap.parse_args()
     import multiprocessing as mp
     import torch
     import zpack_b200
     from zpack_b200 import lib as zlib
     ctx = zpack_b200.Context(0)
+    if a.level >= 3:
+        ctx.set_lz4hc(True)
+    gpu = torch.cuda.get_device_name(0)
+    try:
+        import subprocess
+        gpu += ", power limit " + subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
+                                                 capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        pass
     names = {0: "random", 1: "text", 2: "runs", 3: "records", -1: "mixed"}
     for cls in [int(c) for c in a.classes.split(",")]:
         w = min(os.cpu_count() or 1, 64)
@@ -55,20 +66,31 @@ def main():
         f["dst_off"] = np.arange(n, dtype=np.uint64) * slot
         f["dst_cap"] = cap
         f["method"] = a.method
+        f["level"] = a.level
         d_in = torch.from_numpy(data.reshape(-1)).cuda()
         d_out = torch.empty(n * slot, dtype=torch.uint8, device="cuda")
-        ms = []
+        ms, stages = [], []
         for r in range(a.reps + 1):
             comp, dg, st = ctx.pack_device(d_in, d_in.numel(), d_out, d_out.numel(), f)
             if r:
-                ms.append(ctx.last_kernel_ms()["pack_ms"])
+                k = ctx.last_kernel_ms()
+                ms.append(k["pack_ms"])
+                stages.append((k["pack_blocks_ms"], k["pack_frames_ms"]))
         assert (st == 0).all()
         t = float(np.median(ms))
         unc = n * a.size
-        print(json.dumps({"method": a.method, "class": names[cls], "entries": n, "pack_kernel_ms": round(t, 3),
-                          "uncomp_GBps": round(unc / t / 1e6, 1), "traffic_GBps": round((unc + int(comp.sum())) / t / 1e6, 1),
-                          "ratio_gpu": round(unc / float(comp.sum()), 3), "ratio_reference_level0_sampled": round(unc / ref_comp, 3)}),
-              flush=True)
+        line = {"method": a.method, "level": a.level, "class": names[cls], "entries": n, "pack_kernel_ms": round(t, 3),
+                "uncomp_GBps": round(unc / t / 1e6, 1), "traffic_GBps": round((unc + int(comp.sum())) / t / 1e6, 1),
+                "ratio_gpu": round(unc / float(comp.sum()), 3), "ratio_reference_level0_sampled": round(unc / ref_comp, 3)}
+        if a.level:                   # the stages, and the GPU's level 0 on the same data
+            line["blocks_ms"] = round(float(np.median([x[0] for x in stages])), 3)
+            line["frames_ms"] = round(float(np.median([x[1] for x in stages])), 3)
+            f["level"] = 0
+            comp0, _, st0 = ctx.pack_device(d_in, d_in.numel(), d_out, d_out.numel(), f)
+            assert (st0 == 0).all()
+            line["ratio_gpu_level0"] = round(unc / float(comp0.sum()), 3)
+        line["gpu"] = gpu
+        print(json.dumps(line), flush=True)
     ctx.close()
 
 

@@ -96,6 +96,21 @@ ZPB_DEVINL u32 p2_emit_coop(u8 *dst, u32 op, const u8 *sm, u32 lits, u32 lit, u3
     return op;
 }
 
+// The block into shared memory at window offset D (the caller keeps D congruent to src mod 16): its 16-byte units by one
+// bulk copy that thread 0 issues (completion on the mbarrier `bar`), the unaligned ends by ordinary loads of all
+// `nthreads` threads.  The caller waits on `bar` after a __syncthreads.
+ZPB_DEVINL void p2_stage_block(u8 *sm, u32 D, const u8 *src, u32 n, u32 bar, u32 nthreads) {
+    u32 head = (16u - ((u32)(uintptr_t)src & 15u)) & 15u;
+    if (head > n) head = n;
+    const u32 al = (n - head) & ~15u;
+    if (threadIdx.x == 0) {
+        mbar_arrive_expect_tx(bar, al);
+        for (u32 o = 0; o < al; o += 16384u) bulk_g2s(bar + D + head + o, src + head + o, al - o < 16384u ? al - o : 16384u, bar);
+    }
+    for (u32 i = threadIdx.x; i < head; i += nthreads) sm[D + i] = src[i];
+    for (u32 i = head + al + threadIdx.x; i < n; i += nthreads) sm[D + i] = src[i];
+}
+
 // the warp waits until the token is `want` (true) or the block is given up (false).  Every lane polls, lane 0's view
 // decides: the warp stays converged and the answer is the same in every lane.
 ZPB_DEVINL bool p2_wait(volatile u32 *token, u32 want, volatile u32 *stop) {
@@ -183,18 +198,12 @@ lz4_pack_blocks_body(const u8 *__restrict__ in, const PackBlock *__restrict__ bl
         // ---- the block into shared memory, at the same offset mod 16 as in HBM: 16-byte units by one bulk copy
         // (cp.async.bulk, completion on the mbarrier), the unaligned ends by ordinary loads
         const u32 D = P2_OFF_DATA + ((u32)(uintptr_t)src & 15u);  // block byte i is sm[D + i]
-        u32 head = (16u - ((u32)(uintptr_t)src & 15u)) & 15u;
-        if (head > n) head = n;
-        const u32 al = (n - head) & ~15u;
         if (threadIdx.x == 0) {
             ctl[2] = 0; ctl[3] = 0; ctl[5] = 0;
             for (u32 i = 8; i < 15; ++i) ctl[i] = 0;
             ctl[15] = 1;                             // fits
-            mbar_arrive_expect_tx(bar, al);
-            for (u32 o = 0; o < al; o += 16384u) bulk_g2s(bar + D + head + o, src + head + o, al - o < 16384u ? al - o : 16384u, bar);
         }
-        for (u32 i = threadIdx.x; i < head; i += 32 * P2_WARPS) sm[D + i] = src[i];
-        for (u32 i = head + al + threadIdx.x; i < n; i += 32 * P2_WARPS) sm[D + i] = src[i];
+        p2_stage_block(sm, D, src, n, bar, 32 * P2_WARPS);
         for (u32 i = threadIdx.x; i < (1u << P2_HASH_LOG) / 2; i += 32 * P2_WARPS) reinterpret_cast<u32 *>(sm + tab)[i] = 0;   // position 0 is a harmless candidate: all are verified
         __syncthreads();
         mbar_wait(bar, parity);

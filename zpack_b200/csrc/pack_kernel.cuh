@@ -4,7 +4,7 @@
 // LZ4F_compressBegin / Update / End, externals/lz4/lib/lz4frame.c:598-1022) and the second pass
 // zpack_add_written_file_entry makes for the digest (lib/zpack_write.c:256).  The 64 KB blocks of every LZ4 file of
 // the batch were compressed before this kernel runs, one warp per block, by lz4_pack_blocks_kernel (pack_blocks.cuh)
-// into per-block scratch slots; this kernel lays the frame out — header, block headers, payload from the scratch slot
+// — or, for the HC levels with the context's switch on, by the kernels of lz4hc_blocks.cuh — into per-block scratch slots; this kernel lays the frame out — header, block headers, payload from the scratch slot
 // or the input itself for a block that did not shrink, EndMark — while the same warp streams the file through XXH3.
 //
 // Frames are written with B.Indep = 1 (FLG 0x60), 64 KB blocks, no checksums, no content size:
@@ -17,6 +17,7 @@
 #include "xxh3.cuh"
 #include "lz4_decode.cuh"
 #include "pack_blocks.cuh"
+#include "lz4hc_blocks.cuh"
 #include "zstd_encode.cuh"
 #include "../../include/zpack_b200.h"
 
@@ -26,7 +27,7 @@ __global__ void __launch_bounds__(32 * PK_WARPS)
 lz4_pack_kernel(const u8 *__restrict__ in, u64 in_size, u8 *out, u64 out_size, const zpb_file *__restrict__ files,
                 const u32 *__restrict__ order, u32 n, u32 *counter, u64 *comp_size, u64 *digest, int *status,
                 const u32 *__restrict__ blk_base, const u8 *__restrict__ scratch, const u32 *__restrict__ csize,
-                const u8 *__restrict__ zslot, const u32 *__restrict__ zbody, const u32 *__restrict__ winop) {
+                const u8 *__restrict__ zslot, const u32 *__restrict__ zbody, const u32 *__restrict__ winop, int lz4hc) {
     const int lane = threadIdx.x & 31;
     Group<32> g;
     for (;;) {
@@ -61,7 +62,7 @@ lz4_pack_kernel(const u8 *__restrict__ in, u64 in_size, u8 *out, u64 out_size, c
         } else if (f.method == ZPB_METHOD_LZ4) {
             const u64 nblocks = (f.size + 65535) >> 16;
             if (f.dst_cap < 7 + 4 * nblocks + f.size + 4) st = ZPB_ST_COMPRESS_FAILED;  // LZ4F_compressBound role
-            else if (f.level >= 3) st = ST_NOT_AVAILABLE;   // lz4frame.c:799-807 selects LZ4 HC from level 3 on: not built (SURVEY §8(f) row 2); never a silent downgrade
+            else if (f.level >= 3 && !lz4hc) st = ST_NOT_AVAILABLE;   // lz4frame.c:799-807 selects LZ4 HC from level 3 on: only with the context's HC switch (lz4hc_blocks.cuh); never a silent downgrade
             else {
                 const u8 *src = in + f.src_off;
                 u8 *dst = out + f.dst_off;

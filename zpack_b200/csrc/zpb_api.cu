@@ -87,6 +87,8 @@ struct zpb_ctx {
     int p2_per_sm = 1, pk_per_sm = 1;      // resident CTAs of the two pack kernels
     std::vector<cudaEvent_t> pack_evs;     // three per round: before the block compressor, between, after the framing kernel
     float pack_blocks_ms = 0.f, pack_frames_ms = 0.f;
+    int lz4hc = 0;                         // LZ4 levels >= 3 by the HC compressor (ZPB_LZ4HC=1); off: refused with ZPB_ST_NOT_AVAILABLE
+    DevBuf d_hcrec;                        // pack, HC blocks of a round: per-position match records and parse costs
     // pipelined host path: private sub-contexts (own stream + scratch), one per worker thread
     std::vector<zpb_ctx *> workers;
     // block-sharded path (one large block-independent LZ4 entry): per-KiB XXH3 stripe sums of the last shard
@@ -201,6 +203,11 @@ extern "C" zpb_ctx *zpb_create(int device) {
         delete ctx; return nullptr;
     }
     if (const char *e = getenv("ZPB_PACK_SCRATCH_MB")) ctx->pack_scratch_blocks = std::max<u64>((u64)atoll(e) * 16, 1);
+    if (cudaFuncSetAttribute(lz4hc_match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HC_SMEM) != cudaSuccess) {
+        g_last_error = std::string("LZ4 HC kernel setup failed: ") + cudaGetErrorString(cudaGetLastError());
+        delete ctx; return nullptr;
+    }
+    if (const char *e = getenv("ZPB_LZ4HC")) ctx->lz4hc = atoi(e) != 0;
     return ctx;
 }
 
@@ -214,7 +221,7 @@ extern "C" void zpb_destroy(zpb_ctx *ctx) {
     ctx->d_aux.release(); ctx->d_fe.release(); ctx->d_fb.release(); ctx->d_plist.release();
     ctx->d_glist.release(); ctx->d_fdesc.release(); ctx->d_zlist.release(); ctx->d_zlit.release();
     ctx->d_gather.release(); ctx->d_goff.release(); ctx->h_bounce.release();
-    ctx->d_pblk.release(); ctx->d_pscratch.release(); ctx->d_csize.release();
+    ctx->d_pblk.release(); ctx->d_pscratch.release(); ctx->d_csize.release(); ctx->d_hcrec.release();
     ctx->d_zslot.release(); ctx->d_zseq.release(); ctx->d_zmeta.release(); ctx->d_zelit.release(); ctx->d_zhuf.release(); ctx->d_ztabs.release();
     for (cudaEvent_t e : ctx->pack_evs) cudaEventDestroy(e);
     ctx->d_partials.release(); ctx->d_acc.release();
