@@ -186,7 +186,8 @@ int zpb_pack_host(zpb_ctx *ctx, const uint8_t *h_in, uint64_t in_size, uint8_t *
  * at zpb_create): such files get ZPB_ST_NOT_AVAILABLE.  1: they are compressed by the HC block compressor — hash chains
  * searched up to a level-dependent depth and a cost-based parse per 64 KB block; levels above 12 act as 12.  The frames
  * have the same layout as the fast path's (block-independent, 64 KB blocks).  Levels below 3, zstd and stored files are
- * the same either way.  zpb_pack_host passes the setting on to its worker contexts on every call. */
+ * the same either way.  Like every setting of a context, it reaches the worker contexts of the pipelined host calls
+ * (zpb_unpack_host, zpb_pack_host, zpb_unpack_entry_blocks_host) at the start of every call. */
 int zpb_set_lz4hc(zpb_ctx *ctx, int enabled);
 
 /* last kernel timing (CUDA events on the launching stream), for bench.py's roofline block */
@@ -230,6 +231,7 @@ int zpb_group_unpack_host(zpb_group *g, const uint8_t *h_archive, uint64_t archi
                           uint64_t out_size, const zpb_entry *entries, uint64_t n, int32_t *status, uint64_t *digest);
 int zpb_group_pack_host(zpb_group *g, const uint8_t *h_in, uint64_t in_size, uint8_t *h_out, uint64_t out_size,
                         const zpb_file *files, uint64_t n, uint64_t *comp_size, uint64_t *digest, int32_t *status);
+/* zpb_group_unpack_host and zpb_group_pack_host both record it, on a group of one device too */
 int zpb_group_last_ms(const zpb_group *g, float *ms, int cap);   /* wall time of each device's share of the last call */
 /* pinned host memory for the *_host entry points (pageable buffers make their copies synchronous) */
 void *zpb_host_alloc(uint64_t bytes);

@@ -64,8 +64,6 @@ def main():
     import torch
     import zpack_b200
     from zpack_b200 import container
-    ctx = zpack_b200.Context(0)
-    ctx.set_fast_path(bool(args.fast))
     names = {0: "random", 1: "text", 2: "runs", 3: "records", -1: "mixed"}
     for cls in [int(c) for c in args.classes.split(",")]:
         arch = build(cls, args.entries, args.size, args.independent, 1 if args.method == 'zstd' else 2)
@@ -79,9 +77,11 @@ def main():
                  for c in ([int(x) for x in args.exec_ctas.split(",")] if args.exec_ctas else [0])
                  for ov in ([int(x) for x in args.overlap.split(",")] if args.overlap else [-1])]
         for g, xc, ov in sweep:
-            ctx.set_tuning(group_lanes=g)
             if xc:
-                os.environ["ZPB_EXEC_CTAS"] = str(xc)
+                os.environ["ZPB_EXEC_CTAS"] = str(xc)   # read when a context is created: one context per sweep point
+            ctx = zpack_b200.Context(0)
+            ctx.set_fast_path(bool(args.fast))
+            ctx.set_tuning(group_lanes=g)
             if ov >= 0:
                 ctx.set_overlap(bool(ov))
             ms = []
@@ -104,7 +104,7 @@ def main():
                 ph = ["literals", "seq_tables", "seq_decode", "exec_lit", "exec_par", "exec_order", "hash", "other"]
                 print(json.dumps({"zstd_phase_share": {p: round(a[i] / tot, 3) for i, p in enumerate(ph)},
                                   "Mcycles_per_entry": round(tot / (args.reps + 2) / args.entries / 1e6, 3)}), flush=True)
-    ctx.close()
+            ctx.close()
 
 
 if __name__ == "__main__":

@@ -19,6 +19,31 @@ typedef uint64_t u64;
 
 #define ZPB_DEVINL __device__ __forceinline__
 
+// Slots of a context's counter block (zpb_ctx::d_counter), zeroed before every unpack batch, xxh3 batch and pack round.
+// A "work counter" is the next item a persistent kernel takes; a "length" is a list's size as the kernels appended to it.
+enum CounterSlot : u32 {
+    CNT_WORK = 0,              // work counter of the one-kernel launches: the general kernel, xxh3_kernel, lz4_pack_kernel
+    CNT_GENERAL = 1,           // length of the list the fast path hands to the general kernel
+    CNT_PARSE4_WORK = 2,       // work counter of the split parse walk (lz4_fast_parse4_kernel)
+    CNT_EXEC_WORK = 3,         // work counter of the execute grids over the host's order
+    CNT_GENERAL_WORK = 4,      // work counter of the general kernel over the fast path's list
+    CNT_ZSTD = 5,              // length of the zstd list
+    CNT_ZSTD_WORK = 6,         // work counter of zstd_unpack_kernel
+    CNT_PARSE_HEAVY = 8,       // lengths of the parse lists by weight: heavy, medium (+1), light (+2)
+    CNT_PARSE_MEDIUM = 9,
+    CNT_PARSE_LIGHT = 10,
+    CNT_DEFER_WORK = 11,       // work counter of the execute pass over the entries the early grids put aside
+    CNT_DEFER = 12,            // length of that put-aside list
+    CNT_PARSE_WORK = 13,       // work counter of the first unsplit parse launch
+    CNT_SPLIT_GIVEN_BACK = 14, // statistics: blocks the split walk gave back to the unsplit walk
+    CNT_SPLIT_RETRIES = 15,    // statistics: second attempts of the split walk
+    CNT_LIGHT_FIRST = 17,      // light-list length the first parse launch walked (the last launch walks the rest)
+    CNT_PARSE_LAST_WORK = 18,  // work counter of the last parse launch
+    CNT_PACK_BLOCKS_WORK = 32, // work counter of lz4_pack_blocks_kernel
+    CNT_HC_MATCH_WORK = 48,    // work counter of lz4hc_match_kernel
+    CNT_SLOTS = 64             // size of the block in u32 words
+};
+
 template <int G>
 struct Group {
     static_assert(G >= 4 && G <= 32 && (G & (G - 1)) == 0, "group size");

@@ -98,6 +98,28 @@ struct FastBlock {    // K0 -> K1 -> K2, 32 bytes
     u32 out_size;     // K1 (stored: = bsz)
 };
 
+// Host: the fast path's scratch of entry e, placed at the running totals `slots` (FastBlock slots) and `ndesc` (descriptor
+// words), which grow by what it needs.  An LZ4 frame gets a slot per 64 KB block plus two, and per block FAST_DESC_PER_BLOCK
+// words on top of one per 3 payload bytes (fast_scan_lz4 places block b's descriptors there); an entry the fast path
+// does not take gets nothing.
+inline FastAux fast_entry_layout(const zpb_entry &e, u64 &slots, u64 &ndesc) {
+    u32 ns = 0; u64 nd = 0;
+    if (e.uncomp_size < 0x7fffffffull && e.comp_size) {
+        if (e.method == ZPB_METHOD_NONE) ns = 1;
+        else if (e.method == ZPB_M_LZ4_BLOCK) {
+            ns = 1;
+            nd = ((e.comp_size / 3 + FAST_DESC_PER_BLOCK + 20) + 3) & ~3ull;
+        } else if (e.method == ZPB_METHOD_LZ4) {
+            ns = (u32)(e.uncomp_size >> 16) + 2;
+            nd = ((e.comp_size / 3 + FAST_DESC_PER_BLOCK * ns + 8) + 3) & ~3ull;
+        }
+    }
+    FastAux a;
+    a.desc_base = ndesc; a.slot_base = (u32)slots; a.nslots = ns;
+    slots += ns; ndesc += nd;
+    return a;
+}
+
 // ------------------------------------------------------------------------------------------ K0
 // Returns true when the entry has the shape the fast path handles and the block table is filled.
 __device__ __noinline__ bool fast_scan_lz4(const u8 *src, u64 n, const zpb_entry &e, const FastAux &a,
@@ -194,9 +216,9 @@ lz4_fast_scan_kernel(const u8 *__restrict__ archive, u64 asz, const zpb_entry *_
         status[idx] = st;
         digest[idx] = 0;
     } else if (f.state == FE_GENERAL) {
-        general_list[atomicAdd(&counters[1], 1u)] = idx;
+        general_list[atomicAdd(&counters[CNT_GENERAL], 1u)] = idx;
     } else if (f.state == FE_ZSTD) {
-        zstd_list[atomicAdd(&counters[5], 1u)] = idx;
+        zstd_list[atomicAdd(&counters[CNT_ZSTD], 1u)] = idx;
     } else {
         for (u32 b = 0; b < f.nblocks; ++b)
             if (!(fb[a.slot_base + b].flags & FB_STORED))
@@ -209,7 +231,7 @@ lz4_fast_scan_kernel(const u8 *__restrict__ archive, u64 asz, const zpb_entry *_
                 const u32 peers = __match_any_sync(__activemask(), cls);
                 const int leader = __ffs(peers) - 1;
                 u32 base = 0;
-                if ((int)(threadIdx.x & 31) == leader) base = atomicAdd(&counters[8 + cls], (u32)__popc(peers));
+                if ((int)(threadIdx.x & 31) == leader) base = atomicAdd(&counters[CNT_PARSE_HEAVY + cls], (u32)__popc(peers));
                 base = __shfl_sync(peers, base, leader);
                 parse_list[(u64)cls * plist_cap + base + __popc(peers & ((1u << (threadIdx.x & 31)) - 1u))] = a.slot_base + b;
             }
@@ -427,14 +449,14 @@ lz4_fast_parse_body(const u8 *__restrict__ archive, u64 asz, FastBlock *fb, u32 
                     u32 plist_cap, u32 *counters, u32 *work_counter, u32 *desc, u32 all_lists) {
     // J = 4 walks the heavy list, then the medium one; J = 1 the light one — or, when the batch is so large that even
     // unsplit walks fill the GPU (all_lists bit 0: the host decides), all three, heavy first (K0 sorts blocks by compressed
-    // size).  With the split walk the light list is parsed FIRST (bit 2: remember its length in counters[17]) so that the
+    // size).  With the split walk the light list is parsed FIRST (bit 2: remember its length in CNT_LIGHT_FIRST) so that the
     // execute kernel has entries to start on, and the blocks the split walk gives back, which it appends to the light
-    // list, are walked by a last launch (bit 1: only the items from counters[17] on).
-    const u32 n_heavy = (J == 4 || (all_lists & 1u)) ? counters[8] : 0u;
-    const u32 n_medium = (J == 4 || (all_lists & 1u)) ? counters[9] : 0u;
-    const u32 light_skip = (J == 1 && (all_lists & 2u)) ? counters[17] : 0u;
-    const u32 nitems = J == 4 ? n_heavy + n_medium : n_heavy + n_medium + counters[10] - light_skip;
-    if (J == 1 && (all_lists & 4u) && blockIdx.x == 0 && threadIdx.x == 0) counters[17] = counters[10];
+    // list, are walked by a last launch (bit 1: only the items from CNT_LIGHT_FIRST on).
+    const u32 n_heavy = (J == 4 || (all_lists & 1u)) ? counters[CNT_PARSE_HEAVY] : 0u;
+    const u32 n_medium = (J == 4 || (all_lists & 1u)) ? counters[CNT_PARSE_MEDIUM] : 0u;
+    const u32 light_skip = (J == 1 && (all_lists & 2u)) ? counters[CNT_LIGHT_FIRST] : 0u;
+    const u32 nitems = J == 4 ? n_heavy + n_medium : n_heavy + n_medium + counters[CNT_PARSE_LIGHT] - light_skip;
+    if (J == 1 && (all_lists & 4u) && blockIdx.x == 0 && threadIdx.x == 0) counters[CNT_LIGHT_FIRST] = counters[CNT_PARSE_LIGHT];
     ZPB_DYN_SMEM(k1_smem);
     const u32 lane = threadIdx.x & 31u;
     const u32 sj = lane & (J - 1);                 // this lane's segment
@@ -598,14 +620,14 @@ lz4_fast_parse_body(const u8 *__restrict__ archive, u64 asz, FastBlock *fb, u32 
                         op = 0; nseq = 0; last_ms = 0; had_match = false;
                         mode = K1M_WALK; mptr = 0; msteps = 0; jtok = 0; jop = 0;
                         sg.need(q, q + 1);
-                        if (sj == 3) atomicAdd(&counters[15], 1u);   // statistics: second attempts
+                        if (sj == 3) atomicAdd(&counters[CNT_SPLIT_RETRIES], 1u);   // statistics: second attempts
                     } else {
                         if (sj == 3) {
                             if (failed) {
                                 // still no join, or a genuinely bad block: the unsplit kernel, which runs after this one,
                                 // walks it again from its first byte and has the verdict
-                                parse_list[2ull * plist_cap + atomicAdd(&counters[10], 1u)] = slot;
-                                atomicAdd(&counters[14], 1u);   // statistics: blocks the split walk gave back
+                                parse_list[2ull * plist_cap + atomicAdd(&counters[CNT_PARSE_LIGHT], 1u)] = slot;
+                                atomicAdd(&counters[CNT_SPLIT_GIVEN_BACK], 1u);   // statistics: blocks the split walk gave back
                             } else {
                                 fb[slot].nseq = total;
                                 fb[slot].out_size = out_size;
@@ -1140,7 +1162,7 @@ lz4_fast_exec_kernel(const u8 *__restrict__ archive, u64 asz, u8 *out, const zpb
                 // a block of the sharded path that K1 did not accept: the shard call declines (the caller
                 // re-reads the entry through zpb_unpack_device, whose general decoder has the exact verdict)
                 if (partial) { status[idx] = ST_NOT_AVAILABLE; digest[idx] = 0; }
-                else general_list[atomicAdd(&counters[1], 1u)] = idx;
+                else general_list[atomicAdd(&counters[CNT_GENERAL], 1u)] = idx;
             }
             continue;
         }
@@ -1396,7 +1418,7 @@ lz4_fast_exec_kernel(const u8 *__restrict__ archive, u64 asz, u8 *out, const zpb
             cp_async_wait_all();
             if (lane == 0) {
                 if (partial) { status[idx] = ST_NOT_AVAILABLE; digest[idx] = 0; }
-                else general_list[atomicAdd(&counters[1], 1u)] = idx;
+                else general_list[atomicAdd(&counters[CNT_GENERAL], 1u)] = idx;
             }
             continue;
         }
@@ -1452,5 +1474,3 @@ lz4_fast_exec_kernel(const u8 *__restrict__ archive, u64 asz, u8 *out, const zpb
         }
     }
 }
-typedef void (*fast_exec_fn)(const u8 *__restrict__, u64, u8 *, const zpb_entry *__restrict__, const u32 *__restrict__, u32, u32 *, const FastEntry *__restrict__,
-                             const FastBlock *__restrict__, const u32 *__restrict__, u32 *, u32 *, int *, u64 *, u64 *, u32 *, u32 *, const u32 *);
