@@ -189,6 +189,15 @@ int zpb_pack_host(zpb_ctx *ctx, const uint8_t *h_in, uint64_t in_size, uint8_t *
  * the same either way.  Like every setting of a context, it reaches the worker contexts of the pipelined host calls
  * (zpb_unpack_host, zpb_pack_host, zpb_unpack_entry_blocks_host) at the start of every call. */
 int zpb_set_lz4hc(zpb_ctx *ctx, int enabled);
+/* zstd literals (every zstd level).  0 (the default; env ZPB_ZSTD_ENTROPY=1 turns it on at zpb_create): literals are
+ * Huffman-coded only in blocks whose literal bytes are 0..128, and a block the LZ4 block compressor stored is written as
+ * a Raw_Block.  1: blocks with literal bytes above 128 may also get a code, with FSE-compressed weights, when it saves at
+ * least 1/64 of their literal bytes; and a stored block of 13 bytes or more becomes Compressed_Blocks without sequences
+ * (Huffman-only literals, one per 4 KB window) when that is smaller — the entropy stage zstd level 3 has for data with
+ * few repeats, such as bf16 / fp16 / fp32 / int8 tensors.  Blocks whose literals are bytes 0..128 come out the same
+ * either way, and no frame is larger than with the switch off.  LZ4, LZ4 HC and stored files are not affected.  Like
+ * every setting, it reaches the worker contexts of the pipelined host calls at the start of every call. */
+int zpb_set_zstd_entropy(zpb_ctx *ctx, int enabled);
 
 /* last kernel timing (CUDA events on the launching stream), for bench.py's roofline block */
 int zpb_last_kernel_ms(const zpb_ctx *ctx, float *unpack_ms, float *pack_ms);

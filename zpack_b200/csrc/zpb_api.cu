@@ -70,6 +70,7 @@ struct Settings {
     int fast = 1;                      // scan/parse/exec pipeline for LZ4 + stored entries (ZPB_FAST=0: general kernel only)
     int overlap = 1;                   // ZPB_OVERLAP=0: parse, then execute, on one stream
     int lz4hc = 0;                     // LZ4 levels >= 3 by the HC compressor (ZPB_LZ4HC=1); off: refused with ZPB_ST_NOT_AVAILABLE
+    int zstd_entropy = 0;              // zstd: full-alphabet Huffman literals and literal-only blocks (ZPB_ZSTD_ENTROPY=1); off: today's frames
     u64 pack_scratch_blocks = 16384;   // pack: 64 KB slots per round (ZPB_PACK_SCRATCH_MB, default 1 GiB)
     int arc_dynamic = 1, arc_head_mask = 127;  // copy kernel: chunks drawn from a counter (ZPB_ARC_DYNAMIC=0: fixed deal), head bytes up to the 128-byte grid (ZPB_ARC_HEAD=15: 16-byte grid)
     int arc_ctas_per_sm = 4;           // copy kernel: CTAs per SM (ZPB_ARC_CTAS)
@@ -93,6 +94,7 @@ static Settings settings_from_env() {
     if (const char *s = getenv("ZPB_FAST")) st.fast = atoi(s);
     if (const char *s = getenv("ZPB_OVERLAP")) st.overlap = atoi(s);
     if (const char *s = getenv("ZPB_LZ4HC")) st.lz4hc = atoi(s) != 0;
+    if (const char *s = getenv("ZPB_ZSTD_ENTROPY")) st.zstd_entropy = atoi(s) != 0;
     if (const char *s = getenv("ZPB_PACK_SCRATCH_MB")) st.pack_scratch_blocks = std::max<u64>((u64)atoll(s) * 16, 1);
     if (const char *s = getenv("ZPB_ARC_DYNAMIC")) st.arc_dynamic = atoi(s) != 0;
     if (const char *s = getenv("ZPB_ARC_HEAD")) st.arc_head_mask = atoi(s) == 127 ? 127 : 15;

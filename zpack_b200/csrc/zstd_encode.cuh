@@ -10,7 +10,9 @@
 //   * literals: Huffman-coded in four streams with ONE code per 64 KB block, built from the histogram of all the block's
 //     literals (lengths limited to 11 bits, direct 4-bit weight description); the block's first window with enough
 //     literals carries the tree (Compressed_Literals_Block), the later ones reuse it (Treeless_Literals_Block).  Blocks
-//     whose literals use byte values above 128, short sections and sections that would not shrink stay Raw_Literals.
+//     whose literals use byte values above 128, short sections and sections that would not shrink stay Raw_Literals —
+//     unless the context's entropy switch is on (zpb_set_zstd_entropy): then such blocks get a full-alphabet code with
+//     FSE-compressed weights when it pays, and a block the LZ4 compressor stored becomes literal-only windows (nbSeq = 0).
 //   * sequences: encoded backwards exactly as ZSTD_encodeSequences does (states initialised from the last sequence, extra
 //     bits LL / ML / OF, per earlier sequence the OF, ML, LL state transitions, final states ML, OF, LL, end mark), with
 //     FSE tables fitted to the block's own LL / OF / ML codes: the block's first window with sequences describes them
@@ -20,8 +22,10 @@
 // Raw_Block.
 #pragma once
 #include "common.cuh"
+#include "pack_blocks.cuh"
 
 #ifdef ZPB_SIM
+#include <cmath>
 #define ZE_CONST static const
 #else
 #define ZE_CONST __device__ __constant__
@@ -342,24 +346,90 @@ ZPB_DEVINL bool ze_parse_range(const u8 *lz, u32 begin, u32 end, u32 tail_end, u
 }
 
 // ---- stage B: one Huffman code per 64 KB block, from the histogram of all its literals (huf_compress.c:HUF_buildCTable,
-// HUF_writeCTable).  Lengths are limited to 11 bits by the overflow rule of deflate's gen_bitlen; the description is
-// the direct one (4-bit weights), so only blocks whose literals are bytes 0..128 get a table — text does, binary data
-// keeps raw literals.
+// HUF_writeCTable).  Lengths are limited to 11 bits by the overflow rule of deflate's gen_bitlen.  Blocks whose literals
+// are bytes 0..128 get the direct description (4-bit weights).  Above that only with `full` (the context's entropy
+// switch): the weights are then FSE-compressed, and the caller keeps the table only if ze_huf_settle finds that it pays.
+#define ZE_CARRIER_FIRST 0xFFFFFFFFu   // ZeHuf::carrier: the block's first window with ZE_HUF_MIN literals carries the tree (ze_lit_mode)
 struct ZeHuf {
-    u16 code[ZE_HUF_SYMS + 3];
-    u8 len[ZE_HUF_SYMS + 3];
-    u8 desc[68];          // header byte + weights of symbols 0 .. last-1, two per byte
+    u16 code[256];
+    u8 len[256];
+    u8 desc[128];         // header byte (>= 128: 4-bit weights of symbols 0 .. last-1, two per byte; < 128: bytes of FSE-compressed weights)
     u32 desc_len;         // 0: no table for this block
+    u32 carrier;          // the window that carries the tree, or ZE_CARRIER_FIRST
 };
-ZPB_DEVINL void ze_huf_build(const u32 *hist, ZeHuf &H) {
+
+// FSE-compressed weights, as HUF_compressWeights + FSE_compress_usingCTable_generic write them (huf_compress.c,
+// fse_compress.c): NCount header with table log <= 6, then two interleaved states over the weights from the last to the
+// first.  The decoder counts the weights by where the bitstream ends, so the symbol order, the start of an odd count and
+// the final state flushes (state 2, then state 1, then the end mark) follow the reference exactly.  out[0] = size; returns
+// 1 + size, or 0 when there is no such description: every weight the same (the reference writes none either), or a
+// size of 128 bytes or more, which the header byte cannot express.
+ZPB_DEVINL u32 ze_huf_weights_fse(const u8 *wt, int nw, u8 *out) {
+    u32 cnt[12];
+    for (int s = 0; s < 12; ++s) cnt[s] = 0;
+    for (int i = 0; i < nw; ++i) ++cnt[wt[i]];
+    short norm[12];
+    int last = 0, only = 0;
+    const int log = ze_normalize(cnt, 12, (u32)nw, 6, norm, &last, &only);
+    if (log == 0 || nw <= 2) return 0;
+    u32 buf[32];                                      // the description is built aligned, then copied behind the header byte
+    u8 *b8 = reinterpret_cast<u8 *>(buf);
+    const u32 hs = ze_write_ncount(b8, norm, last, log);
+    ZeSeqTab T;
+    ze_build(T, norm, last + 1, log);
+    ZeBits b;
+    ze_open(b, b8 + hs, b8 + 127, true);
+    const u8 *ip = wt + nw;
+    u32 s1, s2;
+    if (nw & 1) {
+        s1 = ze_init_state(T, *--ip);
+        s2 = ze_init_state(T, *--ip);
+        s1 = ze_encode(b, T, s1, *--ip);
+        ze_flush(b);
+    } else {
+        s2 = ze_init_state(T, *--ip);
+        s1 = ze_init_state(T, *--ip);
+    }
+    while (ip > wt) {                                 // an even number is left: state 2, state 1, ...
+        s2 = ze_encode(b, T, s2, *--ip);
+        ze_flush(b);
+        s1 = ze_encode(b, T, s1, *--ip);
+        ze_flush(b);
+    }
+    ze_add(b, s2 & ((1u << log) - 1u), (u32)log);     // FSE_flushCState: state 2, then state 1
+    ze_flush(b);
+    ze_add(b, s1 & ((1u << log) - 1u), (u32)log);
+    ze_add(b, 1u, 1);                                 // BIT_closeCStream
+    ze_flush_all(b);
+    if (b.ovf) return 0;
+    const u32 size = (u32)(b.p - b8);
+    out[0] = (u8)size;
+    for (u32 i = 0; i < size; ++i) out[1 + i] = b8[i];
+    return 1u + size;
+}
+
+// fixed: bytes the block pays for any table besides its description (6 per window of jump table), for the entropy check.
+ZPB_DEVINL void ze_huf_build(const u32 *hist, ZeHuf &H, bool full = false, u32 fixed = 0) {
     H.desc_len = 0;
+    H.carrier = ZE_CARRIER_FIRST;
     int last = -1, n = 0;
     for (int s = 0; s < 256; ++s) if (hist[s]) { last = s; ++n; }
-    if (n < 2 || last >= (int)ZE_HUF_SYMS) return;
+    if (n < 2 || (last >= (int)ZE_HUF_SYMS && !full)) return;
+    if (last >= (int)ZE_HUF_SYMS) {
+        // No code beats the order-0 entropy: when even that cannot save the 1/64 ze_huf_settle asks for (near-uniform
+        // bytes: random data, most records), skip the build.  The margin keeps the float sum on the safe side, so this
+        // refuses only tables that ze_huf_settle would refuse.
+        u32 total = 0;
+        for (int s = 0; s < 256; ++s) total += hist[s];
+        float bits = 0.f;
+        const float lt = log2f((float)total);
+        for (int s = 0; s < 256; ++s) if (hist[s]) bits += (float)hist[s] * (lt - log2f((float)hist[s]));
+        if (bits * (0.999f / 8.f) - 1.f + (float)(fixed + total / 64u) >= (float)total) return;
+    }
     // leaves by ascending count (insertion sort), then the two-queue construction
-    short order[ZE_HUF_SYMS];
-    u32 cnt[2 * ZE_HUF_SYMS];
-    short parent[2 * ZE_HUF_SYMS];
+    short order[256];
+    u32 cnt[512];
+    short parent[512];
     int m = 0;
     for (int s = 0; s <= last; ++s) {
         if (!hist[s]) continue;
@@ -378,7 +448,7 @@ ZPB_DEVINL void ze_huf_build(const u32 *hist, ZeHuf &H) {
         ++in1;
     }
     const int root = in1 - 1;
-    u8 depth[2 * ZE_HUF_SYMS];
+    u8 depth[512];
     depth[root] = 0;
     for (int i = root - 1; i >= 0; --i) depth[i] = (u8)(depth[parent[i]] + 1);     // parents have larger indices
     // length limit 11: leaves deeper than that are lifted, and for every two of them one shallower leaf goes down a level
@@ -398,10 +468,29 @@ ZPB_DEVINL void ze_huf_build(const u32 *hist, ZeHuf &H) {
         --bl[11];
         overflow -= 2;
     }
+    if (last >= (int)ZE_HUF_SYMS) {
+        // Full alphabets only (the direct description keeps the rule above as it is): with leaves deeper than 12 the rule
+        // leaves the code over-full.  Settle the Kraft sum (in units of 2^-11) exactly: lengthen the longest codes below
+        // 11 while it is over, shorten the longest codes that fit the gap while it is under.
+        int kraft = 0;
+        for (int bits = 1; bits <= 11; ++bits) kraft += bl[bits] << (11 - bits);
+        while (kraft > 2048) {
+            int bits = 10;
+            while (bl[bits] == 0) --bits;
+            --bl[bits]; ++bl[bits + 1];
+            kraft -= 1 << (10 - bits);
+        }
+        while (kraft < 2048) {
+            int bits = 11;
+            while (bl[bits] == 0 || (1 << (11 - bits)) > 2048 - kraft) --bits;
+            --bl[bits]; ++bl[bits - 1];
+            kraft += 1 << (11 - bits);
+        }
+    }
     int maxbits = 11;
     while (bl[maxbits] == 0) --maxbits;
     // lengths back to the symbols: the rarest get the longest codes
-    for (int s = 0; s < (int)ZE_HUF_SYMS + 3; ++s) { H.len[s] = 0; H.code[s] = 0; }
+    for (int s = 0; s < 256; ++s) { H.len[s] = 0; H.code[s] = 0; }
     {
         int i = 0;
         for (int bits = maxbits; bits >= 1; --bits)
@@ -421,8 +510,16 @@ ZPB_DEVINL void ze_huf_build(const u32 *hist, ZeHuf &H) {
         H.code[s] = (u16)(start[w] >> (w - 1));
         start[w] += 1u << (w - 1);
     }
-    // description: 127 + number of weights, then the weights of symbols 0 .. last-1 (the last one is implied)
+    // description: 127 + number of weights, then the weights of symbols 0 .. last-1 (the last one is implied); beyond
+    // 128 weights the FSE-compressed form, which ze_huf_settle has to accept
     const int nw = last;
+    if (last >= (int)ZE_HUF_SYMS) {
+        u8 wt[255];
+        for (int i = 0; i < nw; ++i) wt[i] = H.len[i] ? (u8)(maxbits + 1 - H.len[i]) : (u8)0;
+        H.desc_len = ze_huf_weights_fse(wt, nw, H.desc);
+        H.carrier = 16;                              // none yet
+        return;
+    }
     H.desc[0] = (u8)(127 + nw);
     for (int i = 0; i < nw; i += 2) {
         const u32 w0 = H.len[i] ? (u32)(maxbits + 1 - H.len[i]) : 0u;
@@ -438,6 +535,32 @@ ZPB_DEVINL u32 ze_lit_mode(u32 w, const u32 *lit_n, u32 nwin, bool have_table) {
     if (!have_table || lit_n[w] < ZE_HUF_MIN) return 0;
     for (u32 k = 0; k < w && k < nwin; ++k) if (lit_n[k] >= ZE_HUF_MIN) return 3;
     return 2;
+}
+// The same for a table that names its carrier (full-alphabet tables, ze_huf_settle).
+ZPB_DEVINL u32 ze_lit_mode(u32 w, const u32 *lit_n, u32 nwin, const ZeHuf &H) {
+    if (!H.desc_len) return 0;
+    if (H.carrier == ZE_CARRIER_FIRST) return ze_lit_mode(w, lit_n, nwin, true);
+    if (lit_n[w] < ZE_HUF_MIN || w < H.carrier) return 0;
+    return w == H.carrier ? 2u : 3u;
+}
+
+// A full-alphabet table (ze_huf_build with `full`, symbols above 128) is kept only if it pays: the block's literals,
+// estimated as their coded bits + the description + a 6-byte jump table per window, must save 1/64 against raw
+// literals.  Near-uniform literal bytes (random data, records) then keep raw literals at the cost of the histogram.
+// The tree rides on the first window with ZE_HUF_MIN literals whose section, tree included, is surely smaller than
+// raw (coded bits + one byte per stream + jump table + two bytes of a longer section header): the carrier cannot fall
+// back to raw literals, the windows after it can.  bits[w]: window w's literals coded with H.
+ZPB_DEVINL void ze_huf_settle(ZeHuf &H, const u32 *lit_n, const u32 *bits, u32 nwin) {
+    if (!H.desc_len || H.carrier == ZE_CARRIER_FIRST) return;
+    u32 total = 0;
+    u64 coded = 0;
+    for (u32 w = 0; w < nwin; ++w) { total += lit_n[w]; coded += bits[w]; }
+    u32 carrier = 16;
+    if (coded / 8u + H.desc_len + 6u * nwin + total / 64u < total)
+        for (u32 w = 0; w < nwin && carrier == 16; ++w)
+            if (lit_n[w] >= ZE_HUF_MIN && (bits[w] + 7u) / 8u + 4u + 6u + 2u + H.desc_len < lit_n[w]) carrier = w;
+    H.carrier = carrier;
+    if (carrier == 16) H.desc_len = 0;
 }
 
 // which sequence tables window w uses: 0 predefined, 2 the block's own tables, which this window also describes (it is the
@@ -576,6 +699,82 @@ ZPB_DEVINL u32 ze_emit_range(const u8 *lit, u32 lit_n, const u64 *seq, u32 nseq,
 #define ZE_LOFF(begin, w) ((((begin) + 3u) & ~3u) + 8u * (w))
 #define ZE_META 48u                                   // u32 per block: 16 body sizes | 16 literal counts | 16 sequence counts
 
+// Literal-only blocks (the context's entropy switch on, a block of at least 13 bytes that the LZ4 compressor stored):
+// the same windows as the framing assumes, window w at input offset 4096 w, the last one taking the rest; each becomes
+// a Compressed_Block without sequences whose literals are read in place from the input.  Their bodies sit at
+// ZE_OFF(4096 w, w) with room for 1.25 x the window + 20 bytes, like any other window's.
+ZPB_DEVINL bool ze_lit_only(int entropy, const PackBlock &pb, u32 cs) { return entropy && pb.pad && !cs && pb.len >= 13u; }
+ZPB_DEVINL u32 ze_lit_only_end(u32 len, u32 w, u32 nwin) { return w + 1u == nwin ? len : 4096u * (w + 1u); }
+static_assert(15u * 5144u + 4096u + 1024u + 20u <= ZE_SLOT && 14u * 5144u + 4107u + 1026u + 20u <= ZE_SLOT,
+              "literal-only window bodies fit the block's zstd slot");
+
+// Stage A for window w of block b (t = 16 b + w): the kernel below runs it one thread per window, the CPU emulation in a loop.
+ZPB_DEVINL void ze_stage_parse(u64 t, const u8 *lz_slots, const u32 *csize, const PackBlock *blocks, u32 *winop, u32 *meta, u8 *zlit,
+                               u64 *zseq, int entropy) {
+    const u32 b = (u32)(t >> 4), w = (u32)(t & 15u);
+    const u32 cs = csize[b], len = blocks[b].len;
+    u32 *m = meta + (u64)b * ZE_META;
+    u32 *wo = winop + (u64)b * 17u;
+    u32 lit_n = 0, seq_n = ZE_FAIL;
+    if (ze_lit_only(entropy, blocks[b], cs)) {
+        const u32 nwin = (len - 12u) / 4096u + 1u;
+        seq_n = 0;
+        if (w < nwin) {
+            wo[w] = 4096u * w;
+            lit_n = ze_lit_only_end(len, w, nwin) - 4096u * w;
+        }
+    } else if (blocks[b].pad && cs) {
+        const u32 nwin = (len - 12u) / 4096u + 1u;           // as in pack_blocks.cuh (cs != 0 implies len >= 13)
+        seq_n = 0;
+        if (w < nwin) {
+            const u32 begin = wo[w], end = wo[w + 1u];
+            const u32 tail_end = w + 1u == nwin ? cs : end;
+            if (!(begin <= end && tail_end <= cs && end <= tail_end) ||
+                !ze_parse_range(lz_slots + ((u64)b << 16), begin, end, tail_end, zlit + (u64)b * ZE_LITSLOT + ZE_LOFF(begin, w),
+                                zseq + t * ZE_WIN_SEQ, ZE_WIN_SEQ, &lit_n, &seq_n))
+                seq_n = ZE_FAIL;
+        }
+    }
+    m[16u + w] = lit_n;
+    m[32u + w] = seq_n;
+}
+
+// Stage C for window w of block b (t = 16 b + w), likewise.
+ZPB_DEVINL void ze_stage_encode(u64 t, const u8 *in, const u32 *csize, const PackBlock *blocks, const u32 *winop, u32 *meta, const u8 *zlit,
+                                const u64 *zseq, const ZeHuf *hufs, const ZeBlockTabs *tabs, u8 *zslot, int entropy, const ZeTables &T) {
+    const u32 b = (u32)(t >> 4), w = (u32)(t & 15u);
+    u32 *m = meta + (u64)b * ZE_META;
+    u32 z = 0;
+    if (ze_lit_only(entropy, blocks[b], csize[b])) {
+        const u32 len = blocks[b].len, nwin = (len - 12u) / 4096u + 1u;
+        const ZeHuf &H = hufs[b];
+        if (!H.desc_len) z = ZE_FAIL;
+        else if (w < nwin) {
+            const u32 begin = 4096u * w, n = ze_lit_only_end(len, w, nwin) - begin;
+            z = ze_emit_range(in + blocks[b].src_off + begin, n, nullptr, 0, ze_lit_mode(w, m + 16u, nwin, H), H,
+                              zslot + (u64)b * ZE_SLOT + ZE_OFF(begin, w), n + (n >> 2) + 20u, T, 0, tabs[b]);
+        }
+    } else if (blocks[b].pad && csize[b]) {
+        const u32 nwin = (blocks[b].len - 12u) / 4096u + 1u;
+        if (w < nwin) {
+            const u32 begin = winop[(u64)b * 17u + w], end = winop[(u64)b * 17u + w + 1u];
+            const u32 tail_end = w + 1u == nwin ? csize[b] : end;
+            const u32 seq_n = m[32u + w];
+            if (seq_n == ZE_FAIL) z = ZE_FAIL;
+            else {
+                const ZeHuf &H = hufs[b];
+                const ZeBlockTabs &B = tabs[b];
+                const u32 mode = ze_lit_mode(w, m + 16u, nwin, H);
+                const u32 seqmode = ze_seq_mode(w, m + 32u, nwin, B.valid != 0);
+                z = ze_emit_range(zlit + (u64)b * ZE_LITSLOT + ZE_LOFF(begin, w), m[16u + w], zseq + t * ZE_WIN_SEQ, seq_n, mode, H,
+                                  zslot + (u64)b * ZE_SLOT + ZE_OFF(begin, w), (tail_end - begin) + ((tail_end - begin) >> 2) + 20u, T,
+                                  seqmode, B);
+            }
+        }
+    } else if (w == 0) z = ZE_FAIL;
+    m[w] = z;
+}
+
 #ifndef ZPB_SIM
 // Three launches per round, all over the blocks the host marked (PackBlock::pad != 0: they belong to a
 // ZPACK_COMPRESSION_ZSTD file).  meta = ZE_META words per block, winop = 17 window offsets per block.
@@ -583,40 +782,25 @@ ZPB_DEVINL u32 ze_emit_range(const u8 *lit, u32 lit_n, const u64 *seq, u32 nseq,
 // A: one THREAD per 4 KB window of the block compressor (its payload offsets come from lz4_pack_blocks_kernel: winop):
 //    the window's LZ4 sequences -> staged literal bytes + sequence records.  Each walk is serial and latency-bound, so the
 //    kernel relies on the number of windows in flight (16 per block, every block of the round at once), not on staging.
+//    A literal-only block (entropy switch) needs no walk: its windows' offsets go to winop, their sizes to meta.
 __global__ void __launch_bounds__(128)
 zstd_parse_windows_kernel(const u8 *__restrict__ lz_slots, const u32 *__restrict__ csize, const PackBlock *__restrict__ blocks,
-                          const u32 *__restrict__ winop, u32 nblocks, u32 *meta, u8 *zlit, u64 *zseq) {
+                          u32 *winop, u32 nblocks, u32 *meta, u8 *zlit, u64 *zseq, int entropy) {
     const u64 nwork = (u64)nblocks * 16u;
-    for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < nwork; t += (u64)gridDim.x * blockDim.x) {
-        const u32 b = (u32)(t >> 4), w = (u32)(t & 15u);
-        const u32 cs = csize[b], len = blocks[b].len;
-        u32 *m = meta + (u64)b * ZE_META;
-        const u32 *wo = winop + (u64)b * 17u;
-        u32 lit_n = 0, seq_n = ZE_FAIL;
-        if (blocks[b].pad && cs) {
-            const u32 nwin = (len - 12u) / 4096u + 1u;           // as in pack_blocks.cuh (cs != 0 implies len >= 13)
-            seq_n = 0;
-            if (w < nwin) {
-                const u32 begin = wo[w], end = wo[w + 1u];
-                const u32 tail_end = w + 1u == nwin ? cs : end;
-                if (!(begin <= end && tail_end <= cs && end <= tail_end) ||
-                    !ze_parse_range(lz_slots + ((u64)b << 16), begin, end, tail_end, zlit + (u64)b * ZE_LITSLOT + ZE_LOFF(begin, w),
-                                    zseq + t * ZE_WIN_SEQ, ZE_WIN_SEQ, &lit_n, &seq_n))
-                    seq_n = ZE_FAIL;
-            }
-        }
-        m[16u + w] = lit_n;
-        m[32u + w] = seq_n;
-    }
+    for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < nwork; t += (u64)gridDim.x * blockDim.x)
+        ze_stage_parse(t, lz_slots, csize, blocks, winop, meta, zlit, zseq, entropy);
 }
 
 // B: one warp per block: histograms of the block's staged literals and of its sequence codes in shared memory; lane 0
-// builds the Huffman code and the three FSE tables.
+// builds the Huffman code and the three FSE tables.  A full-alphabet code (entropy switch, literals above 128) is then
+// priced window by window by the whole warp, and ze_huf_settle keeps it or not.
 __global__ void __launch_bounds__(128)
-zstd_huf_tables_kernel(const PackBlock *__restrict__ blocks, const u32 *__restrict__ csize, const u32 *__restrict__ winop, u32 nblocks,
-                       const u32 *__restrict__ meta, const u8 *__restrict__ zlit, const u64 *__restrict__ zseq, ZeHuf *hufs,
-                       ZeBlockTabs *tabs) {
+zstd_huf_tables_kernel(const u8 *__restrict__ in, const PackBlock *__restrict__ blocks, const u32 *__restrict__ csize,
+                       const u32 *__restrict__ winop, u32 nblocks, const u32 *__restrict__ meta, const u8 *__restrict__ zlit,
+                       const u64 *__restrict__ zseq, ZeHuf *hufs, ZeBlockTabs *tabs, int entropy) {
     __shared__ u32 hist_all[4][256 + 128];
+    __shared__ u32 wbits_all[4][16];
+    __shared__ u8 lens_all[4][256];
     const u32 lane = threadIdx.x & 31u, wp = threadIdx.x >> 5;
     u32 *hist = hist_all[wp];
     u32 *hll = hist + 256, *hof = hist + 256 + 36, *hml = hist + 256 + 36 + 32;      // 36 + 32 + 53 code counters
@@ -625,13 +809,29 @@ zstd_huf_tables_kernel(const PackBlock *__restrict__ blocks, const u32 *__restri
         for (u32 i = lane; i < 256 + 128; i += 32) hist[i] = 0;
         __syncwarp();
         u32 total = 0, nseq = 0;
-        bool ok = blocks[b].pad && csize[b];
-        if (ok) {
-            const u32 nwin = (blocks[b].len - 12u) / 4096u + 1u;
+        const bool lit_only = ze_lit_only(entropy, blocks[b], csize[b]);
+        const u32 nwin = (blocks[b].len - 12u) / 4096u + 1u;
+        const u8 *blk_in = in + blocks[b].src_off, *blk_lit = zlit + (u64)b * ZE_LITSLOT;
+        auto lits = [&](u32 w) { const u32 o = winop[(u64)b * 17u + w]; return lit_only ? blk_in + o : blk_lit + ZE_LOFF(o, w); };
+        bool ok = blocks[b].pad && (csize[b] || lit_only);
+        if (lit_only) {             // the whole block, contiguous in the input: 16-byte loads between the unaligned ends
+            const u32 len = blocks[b].len;
+            const u32 head = min((16u - (u32)((uintptr_t)blk_in & 15u)) & 15u, len), nv = (len - head) >> 4;
+            const uint4 *v = reinterpret_cast<const uint4 *>(blk_in + head);
+            for (u32 i = lane; i < head; i += 32) atomicAdd(&hist[blk_in[i]], 1u);
+            for (u32 i = lane; i < nv; i += 32) {
+                const uint4 x = v[i];
+                const u32 wd[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+                for (int k = 0; k < 16; ++k) atomicAdd(&hist[(wd[k >> 2] >> (8 * (k & 3))) & 0xFFu], 1u);
+            }
+            for (u32 i = head + (nv << 4) + lane; i < len; i += 32) atomicAdd(&hist[blk_in[i]], 1u);
+            total = len;
+        } else if (ok) {
             for (u32 w = 0; w < nwin; ++w) {
                 if (m[32u + w] == ZE_FAIL) { ok = false; break; }
                 const u32 n = m[16u + w];
-                const u8 *p = zlit + (u64)b * ZE_LITSLOT + ZE_LOFF(winop[(u64)b * 17u + w], w);
+                const u8 *p = lits(w);
                 for (u32 i = lane; i < n; i += 32) atomicAdd(&hist[p[i]], 1u);
                 total += n;
                 const u32 ns = m[32u + w];
@@ -657,46 +857,42 @@ zstd_huf_tables_kernel(const PackBlock *__restrict__ blocks, const u32 *__restri
             }
             if (lane == 0) B.valid = fit ? 1u : 0u;
         } else if (lane == 3) {
-            if (ok && total >= 256u) ze_huf_build(hist, hufs[b]);
-            else hufs[b].desc_len = 0;
+            if (ok && total >= 256u) ze_huf_build(hist, hufs[b], entropy != 0, 6u * nwin);
+            else { hufs[b].desc_len = 0; hufs[b].carrier = ZE_CARRIER_FIRST; }
+        }
+        __syncwarp();
+        const int settle = __shfl_sync(0xffffffffu, (int)(lane == 3 && hufs[b].desc_len && hufs[b].carrier != ZE_CARRIER_FIRST), 3);
+        if (settle) {
+            u32 *wbits = wbits_all[wp];
+            u8 *lens = lens_all[wp];
+            for (u32 i = lane; i < 256; i += 32) lens[i] = hufs[b].len[i];
+            __syncwarp();
+            for (u32 w = 0; w < nwin; ++w) {
+                const u32 n = m[16u + w];
+                const u8 *p = lits(w);
+                u32 bits = 0;
+                for (u32 i = lane; i < n; i += 32) bits += lens[p[i]];
+                for (int d = 16; d; d >>= 1) bits += __shfl_xor_sync(0xffffffffu, bits, d);
+                if (lane == 0) wbits[w] = bits;
+            }
+            __syncwarp();
+            if (lane == 0) ze_huf_settle(hufs[b], m + 16u, wbits, nwin);
         }
         __syncwarp();
     }
 }
 
 // C: one thread per window again: the window's sub-block body.  meta[w]: body size (0: none, ZE_FAIL: the
-// block is stored raw).
+// block is stored raw).  A literal-only block without a table is stored without encoding anything.
 __global__ void __launch_bounds__(128)
-zstd_encode_windows_kernel(const u32 *__restrict__ csize, const PackBlock *__restrict__ blocks, const u32 *__restrict__ winop, u32 nblocks,
-                           u32 *meta, const u8 *__restrict__ zlit, const u64 *__restrict__ zseq, const ZeHuf *__restrict__ hufs,
-                           const ZeBlockTabs *__restrict__ tabs, u8 *zslot) {
+zstd_encode_windows_kernel(const u8 *__restrict__ in, const u32 *__restrict__ csize, const PackBlock *__restrict__ blocks,
+                           const u32 *__restrict__ winop, u32 nblocks, u32 *meta, const u8 *__restrict__ zlit, const u64 *__restrict__ zseq,
+                           const ZeHuf *__restrict__ hufs, const ZeBlockTabs *__restrict__ tabs, u8 *zslot, int entropy) {
     __shared__ ZeTables T;
     if (threadIdx.x == 0) ze_build_tables(T);
     __syncthreads();
     const u64 nwork = (u64)nblocks * 16u;
-    for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < nwork; t += (u64)gridDim.x * blockDim.x) {
-        const u32 b = (u32)(t >> 4), w = (u32)(t & 15u);
-        u32 *m = meta + (u64)b * ZE_META;
-        u32 z = 0;
-        if (blocks[b].pad && csize[b]) {
-            const u32 nwin = (blocks[b].len - 12u) / 4096u + 1u;
-            if (w < nwin) {
-                const u32 begin = winop[(u64)b * 17u + w], end = winop[(u64)b * 17u + w + 1u];
-                const u32 tail_end = w + 1u == nwin ? csize[b] : end;
-                const u32 seq_n = m[32u + w];
-                if (seq_n == ZE_FAIL) z = ZE_FAIL;
-                else {
-                    const ZeHuf &H = hufs[b];
-                    const ZeBlockTabs &B = tabs[b];
-                    const u32 mode = ze_lit_mode(w, m + 16u, nwin, H.desc_len != 0);
-                    const u32 seqmode = ze_seq_mode(w, m + 32u, nwin, B.valid != 0);
-                    z = ze_emit_range(zlit + (u64)b * ZE_LITSLOT + ZE_LOFF(begin, w), m[16u + w], zseq + t * ZE_WIN_SEQ, seq_n, mode, H,
-                                      zslot + (u64)b * ZE_SLOT + ZE_OFF(begin, w), (tail_end - begin) + ((tail_end - begin) >> 2) + 20u, T,
-                                      seqmode, B);
-                }
-            }
-        } else if (w == 0) z = ZE_FAIL;
-        m[w] = z;
-    }
+    for (u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x; t < nwork; t += (u64)gridDim.x * blockDim.x)
+        ze_stage_encode(t, in, csize, blocks, winop, meta, zlit, zseq, hufs, tabs, zslot, entropy, T);
 }
 #endif

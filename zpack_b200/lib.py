@@ -56,7 +56,7 @@ EXPORTS = [
     "zpb_abi_version", "zpb_create", "zpb_destroy", "zpb_last_error", "zpb_device_info",
     "zpb_launch_count", "zpb_unpack_device", "zpb_unpack_host", "zpb_xxh3_device", "zpb_xxh3_host",
     "zpb_pack_bound", "zpb_pack_device", "zpb_pack_host", "zpb_last_kernel_ms", "zpb_last_pack_stage_ms", "zpb_set_tuning",
-    "zpb_last_stage_ms", "zpb_set_fast_path", "zpb_set_overlap", "zpb_set_lz4hc", "zpb_last_zstd_ms",
+    "zpb_last_stage_ms", "zpb_set_fast_path", "zpb_set_overlap", "zpb_set_lz4hc", "zpb_set_zstd_entropy", "zpb_last_zstd_ms",
     "zpb_lz4_frame_index", "zpb_unpack_blocks_device", "zpb_blocks_digest", "zpb_last_chain_ms",
     "zpb_unpack_entry_blocks_host", "zpb_device_count",
     "zpb_archive_open_device", "zpb_archive_build_device", "zpb_copy_entries_device", "zpb_last_archive_ms",
@@ -104,6 +104,7 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.zpb_set_fast_path.argtypes = [vp, C.c_int]
     lib.zpb_set_overlap.argtypes = [vp, C.c_int]
     lib.zpb_set_lz4hc.argtypes = [vp, C.c_int]
+    lib.zpb_set_zstd_entropy.argtypes = [vp, C.c_int]
     lib.zpb_last_zstd_ms.argtypes = [vp, C.POINTER(C.c_float)]
     lib.zpb_lz4_frame_index.argtypes = [vp, u64, u64, vp, u64, u64p, C.POINTER(C.c_uint32), u64p]
     lib.zpb_unpack_blocks_device.argtypes = [vp, vp, u64, vp, u64, vp, u64, C.c_uint32, u64, i32p, vp]
@@ -268,6 +269,12 @@ class Context:
         """True: LZ4 files of level >= 3 are compressed by the HC block compressor (levels above 12 act as 12);
         False (the default unless ZPB_LZ4HC=1 was set when the context was created): they get ST_NOT_AVAILABLE."""
         self._check(self.lib.zpb_set_lz4hc(self.h, int(enabled)))
+
+    def set_zstd_entropy(self, enabled: bool):
+        """True: zstd files also Huffman-code literals with byte values above 128 (FSE-compressed weights) where that
+        pays, and blocks the LZ4 block compressor stores become Huffman-only Compressed_Blocks where that is smaller.
+        False (the default unless ZPB_ZSTD_ENTROPY=1 was set when the context was created): today's frames."""
+        self._check(self.lib.zpb_set_zstd_entropy(self.h, int(enabled)))
 
     def last_stage_ms(self):
         a = (C.c_float * 4)()
