@@ -114,15 +114,20 @@ int zpb_unpack_host(zpb_ctx *ctx, const uint8_t *h_archive, uint64_t archive_siz
  * (FLG B.Indep = 1 — what zpb_pack_* writes; the reference reader accepts both modes,
  * /root/reference/externals/lz4/lib/lz4frame.c:1151,1676) is decoded one warp per block, and a contiguous
  * run of its blocks can be given to each GPU.  Replaces, for such an entry, the LZ4F_decompress loop and the
- * XXH3_64bits pass of zpack_read_file (/root/reference/lib/zpack_read.c:396-468).  Reference-written
- * (block-linked) and zstd entries are one dependency chain each and stay on zpb_unpack_*. */
+ * XXH3_64bits pass of zpack_read_file (/root/reference/lib/zpack_read.c:396-468).  A large zstd entry written by
+ * zpb_pack_* (one frame per 64 KB, zpb_zstd_frame_index) is decoded the same way, one warp per frame.  Reference-written
+ * LZ4 (block-linked) and zstd (one frame) entries are one dependency chain each and stay on zpb_unpack_*. */
 typedef struct zpb_block {
     uint64_t src_off;      /* archive offset of the block payload (after its 4-byte header) */
     uint32_t comp_size;    /* payload bytes                                                */
     uint32_t flags;        /* ZPB_BLK_STORED: payload is the data itself (header bit 31)    */
 } zpb_block;
 #define ZPB_BLK_STORED 1u
-#define ZPB_INDEX_UNSUPPORTED 1   /* zpb_lz4_frame_index: not a single checksum-free B.Indep frame of 64 KB blocks */
+#define ZPB_BLK_ZSTD   2u  /* zpb_zstd_frame_index: the "block" is one whole zstd frame (src_off = its magic number) */
+#define ZPB_INDEX_UNSUPPORTED 1   /* the index functions: the entry does not have the shape the block path takes */
+/* Decoded size from which zpb_pack_* writes a zstd file as one frame per 64 KB of input (zpb_zstd_frame_index), and
+ * from which the drop-in reader sends LZ4 and zstd entries to the block path. */
+#define ZPB_ZSTD_FRAMED_MIN (4ull << 20)
 
 /* Host-side framing walk (no codec work): header checks of LZ4F_decodeHeader (lz4frame.c:1113-1205) and the
  * block-header chain (lz4frame.c:1503-1531) of the frame at h_frame[0..comp_size).  `archive_off` is added to
@@ -132,7 +137,21 @@ typedef struct zpb_block {
 int zpb_lz4_frame_index(const uint8_t *h_frame, uint64_t comp_size, uint64_t archive_off, zpb_block *blocks,
                         uint64_t cap, uint64_t *n_blocks, uint32_t *block_size, uint64_t *content_size);
 
+/* The zstd counterpart: a zstd entry of at least ZPB_ZSTD_FRAMED_MIN bytes written by zpb_pack_* is a sequence of
+ * independent frames, frame k holding decoded bytes [65536 k, 65536 (k + 1)).  Walks the frame headers
+ * (zstd_compression_format.md, Frame_Header) and each frame's 3-byte block-header chain, and writes up to `cap`
+ * entries, one per frame: src_off = archive_off + where the frame starts, comp_size = the frame's bytes, flags =
+ * ZPB_BLK_ZSTD; always sets *n_frames and *content_size (the sum of the frames' Frame_Content_Size).  Only that shape
+ * is taken: every frame has a Frame_Content_Size, no dictionary ID and no checksum; every frame but the last holds
+ * exactly 65 536 bytes and the last 1 to 65 536; the frames end exactly at comp_size.  Anything else — skippable
+ * frames, one frame of more than 64 KB (what the reference's writer produces), truncation, trailing bytes — returns
+ * ZPB_INDEX_UNSUPPORTED (use zpb_unpack_* instead).  ZPB_E_ARG on a null pointer. */
+int zpb_zstd_frame_index(const uint8_t *h_entry, uint64_t comp_size, uint64_t archive_off, zpb_block *frames,
+                         uint64_t cap, uint64_t *n_frames, uint64_t *content_size);
+
 /* Decode blocks[0..n) — a contiguous run of one entry's blocks — into d_out + k * block_size.
+ * The run is either LZ4 blocks (zpb_lz4_frame_index) or zstd frames (zpb_zstd_frame_index, flags ZPB_BLK_ZSTD, one
+ * warp per frame); mixing the two in one call is ZPB_E_ARG.
  * shard_uncomp_size = decoded bytes of the run: every block but the run's last must decode to exactly
  * block_size (LZ4F writers fill blocks, lz4frame.c:873-882); only the entry's last shard may end short.
  * *status: 0, ZPB_ST_OFFSET_INVALID, or ZPB_ST_NOT_AVAILABLE = this path declines the shard (a block is
@@ -150,11 +169,12 @@ int zpb_unpack_blocks_device(zpb_ctx *ctx, const uint8_t *d_archive, uint64_t ar
  * and the merge (xxhash.h:3701-3747) run there. */
 int zpb_blocks_digest(zpb_ctx *ctx, const uint64_t *acc_in, uint64_t *acc_out, uint64_t shard_pos,
                       uint64_t total_size, const uint8_t *d_out, uint64_t *digest, void *stream);
-/* zpack_read_file for ONE large block-independent LZ4 entry with host buffers: frame index, then chunks of
- * blocks pipelined over the context's worker streams (H2D / decode / chain / D2H overlap), the XXH3 state
- * relayed chunk to chunk.  Returns ZPB_OK with *status = the entry's zpack_result, or ZPB_INDEX_UNSUPPORTED
- * when the entry is not eligible (linked blocks, checksums, sizes that do not add up, a block the fast
- * kernels decline) — the caller then uses zpb_unpack_host, which decodes anything.  flags: ZPB_F_*. */
+/* zpack_read_file for ONE large block-independent LZ4 entry, or one zstd entry of 64 KB frames, with host buffers:
+ * frame index (chosen by the entry's magic number), then chunks of blocks / frames pipelined over the context's worker
+ * streams (H2D / decode / chain / D2H overlap), the XXH3 state relayed chunk to chunk.  Returns ZPB_OK with *status =
+ * the entry's zpack_result, or ZPB_INDEX_UNSUPPORTED when the entry is not eligible (linked blocks, checksums, a zstd
+ * entry that is not 64 KB frames, sizes that do not add up, a block or frame the kernels decline) — the caller then
+ * uses zpb_unpack_host, which decodes anything.  flags: ZPB_F_*. */
 int zpb_unpack_entry_blocks_host(zpb_ctx *ctx, const uint8_t *h_entry, uint64_t comp_size, uint8_t *h_out,
                                  uint64_t out_cap, uint64_t uncomp_size, uint64_t expect_hash, uint32_t flags,
                                  int32_t *status, uint64_t *digest);
@@ -167,7 +187,9 @@ int zpb_xxh3_device(zpb_ctx *ctx, const uint8_t *d_data, const uint64_t *offsets
 int zpb_xxh3_host(zpb_ctx *ctx, const uint8_t *h_data, uint64_t length, uint64_t *digest);
 
 /* pack ------------------------------------------------------------------------------------ */
-/* worst-case output bytes for one file (LZ4: frame header + per-block headers + EndMark) */
+/* worst-case output bytes for one file (LZ4: frame header + per-block headers + EndMark; zstd below
+ * ZPB_ZSTD_FRAMED_MIN: frame header + per-block headers; zstd from ZPB_ZSTD_FRAMED_MIN on: per 64 KB a frame header of
+ * at most 7 bytes, a 3-byte block header and the payload) */
 uint64_t zpb_pack_bound(uint32_t method, uint64_t size);
 
 /* Compress n files that are resident in HBM into their slots; returns per-file compressed

@@ -76,6 +76,9 @@ static_assert((FAST_RING & FAST_RMASK) == 0 && FAST_RING % 1024u == 0, "output r
 // zpb_entry.reserved = index of the block's first KiB in the per-KiB XXH3 stripe-sum array; such
 // "partial" entries emit stripe sums instead of a digest (the chain is run by xxh3_chain_kernel).
 #define ZPB_M_LZ4_BLOCK   0x102u
+// Likewise one whole zstd frame of an entry written as 64 KB frames (zpb_zstd_frame_index): queued for the zstd kernel,
+// whose ZsPartialHasher instantiation leaves the frame's stripe sums at `reserved` the same way.
+#define ZPB_M_ZSTD_FRAME  0x103u
 #define ZPB_F_STORED_BLK  0x100u
 #define FE_LINK_NONE    0u
 #define FE_LINK_WINDOW  1u   // blocks of the frame share the 64 KB window (B.Indep = 0)
@@ -207,7 +210,7 @@ lz4_fast_scan_kernel(const u8 *__restrict__ archive, u64 asz, const zpb_entry *_
             f.linked = FE_LINK_PARTIAL;
             f.state = FE_FAST;
         }
-    } else if (e.method == ZPB_METHOD_ZSTD) {
+    } else if (e.method == ZPB_METHOD_ZSTD || e.method == ZPB_M_ZSTD_FRAME) {
         f.state = FE_ZSTD;                                     // guards passed: the zstd kernel decodes it
     } else {
         f.state = FE_GENERAL;                                  // unknown method: the general kernel answers

@@ -23,6 +23,13 @@
 
 #define PK_WARPS 4
 
+// zstd: frame header 14 + per 64 KB block a 3-byte header + at most the raw payload; from ZPB_ZSTD_FRAMED_MIN on, one
+// frame per 64 KB block: a header of at most 7 bytes + a 3-byte block header + at most the raw payload
+__host__ __device__ inline u64 zstd_pack_bound(u64 size) {
+    const u64 nb = size ? (size + 65535) >> 16 : 1;
+    return size >= ZPB_ZSTD_FRAMED_MIN ? 10 * nb + size : 14 + 3 * nb + size;
+}
+
 __global__ void __launch_bounds__(32 * PK_WARPS)
 lz4_pack_kernel(const u8 *__restrict__ in, u64 in_size, u8 *out, u64 out_size, const zpb_file *__restrict__ files,
                 const u32 *__restrict__ order, u32 n, u32 *counter, u64 *comp_size, u64 *digest, int *status,
@@ -102,25 +109,38 @@ lz4_pack_kernel(const u8 *__restrict__ in, u64 in_size, u8 *out, u64 out_size, c
         } else if (f.method == ZPB_METHOD_ZSTD) {
             // A zstd frame of 64 KB blocks (zstd_compression_format.md:320-404): Compressed_Blocks whose bodies
             // zstd_encode_blocks_kernel built from the block compressor's matches (raw literals + predefined-mode FSE
-            // sequences), Raw_Blocks where that did not shrink the block.
+            // sequences), Raw_Blocks where that did not shrink the block.  From ZPB_ZSTD_FRAMED_MIN on, every 64 KB
+            // block is a frame of its own (the same blocks behind a single-segment header): the frames say what the
+            // blocks already are — independent — so a reader can decode them in parallel (zpb_zstd_frame_index).
             const u64 nblocks = f.size ? (f.size + 65535) >> 16 : 1;
-            if (f.dst_cap < 14 + 3 * nblocks + f.size) st = ZPB_ST_COMPRESS_FAILED;
+            const bool framed = f.size >= ZPB_ZSTD_FRAMED_MIN;
+            if (f.dst_cap < zstd_pack_bound(f.size)) st = ZPB_ST_COMPRESS_FAILED;
             else {
                 const u8 *src = in + f.src_off;
                 u8 *dst = out + f.dst_off;
                 const u32 b0 = blk_base[idx];
-                if (lane == 0) {
+                if (lane == 0 && !framed) {
                     // magic; FHD: 8-byte frame content size, no single-segment, no checksum, no dictionary; window 128 KB
                     dst[0] = 0x28; dst[1] = 0xB5; dst[2] = 0x2F; dst[3] = 0xFD; dst[4] = 0xC0; dst[5] = 0x38;
                     for (int k = 0; k < 8; ++k) dst[6 + k] = (u8)(f.size >> (8 * k));
                 }
-                u64 op = 14;
+                u64 op = framed ? 0 : 14;
                 Xxh3Stream<32> hs;
                 hs.init(src, f.size, g);
                 for (u64 b = 0; b < nblocks; ++b) {
                     const u32 blen = (u32)(f.size - (b << 16) < 65536 ? f.size - (b << 16) : 65536);
                     const u64 bb = b0 + b;
-                    const bool last_block = b + 1 == nblocks;
+                    const bool last_block = framed || b + 1 == nblocks;
+                    if (framed) {
+                        // magic; FHD: single segment (the window is the content), no checksum, no dictionary, and the
+                        // smallest Frame_Content_Size field: 1 byte up to 255, else 2 bytes holding size - 256
+                        if (lane == 0) {
+                            dst[op] = 0x28; dst[op + 1] = 0xB5; dst[op + 2] = 0x2F; dst[op + 3] = 0xFD;
+                            if (blen < 256) { dst[op + 4] = 0x20; dst[op + 5] = (u8)blen; }
+                            else { dst[op + 4] = 0x60; dst[op + 5] = (u8)(blen - 256); dst[op + 6] = (u8)((blen - 256) >> 8); }
+                        }
+                        op += blen < 256 ? 6 : 7;
+                    }
                     // the block's windows: lanes 0-15 look at one body size each; any failure, or bodies that are not
                     // smaller than the block, and it is stored raw
                     u32 zw = f.size && lane < 16 ? zbody[bb * ZE_ZBODY + lane] : 0u;

@@ -128,6 +128,7 @@ struct zpb_ctx {
     DevBuf d_aux, d_fe, d_fb, d_plist, d_glist, d_fdesc;
     DevBuf d_zlist, d_zlit;  // zstd work list, per-warp literal buffers
     int zs_grid = 0;         // persistent grid of zstd_unpack_kernel (CTAs)
+    int zs_grid_part = 0;    // the same for its frame-parallel instantiation (zpb_unpack_blocks_device)
     float zstd_ms = 0.f;
     Event evs[6];
     // the execute kernel runs on its own stream so that it overlaps the tail of the parse kernel
@@ -230,15 +231,18 @@ extern "C" zpb_ctx *zpb_create(int device) {
         return nullptr;
     }
     {
-        int per_sm = 0;
+        int per_sm = 0, per_sm_part = 0;
         const int smem = (int)(ZS_WARPS * sizeof(ZstdShared));
-        if (cudaFuncSetAttribute(zstd_unpack_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess ||
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, zstd_unpack_kernel, ZS_WARPS * 32, smem) != cudaSuccess ||
-            per_sm < 1) {
+        if (cudaFuncSetAttribute(zstd_unpack_kernel<ZsHasher>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess ||
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, zstd_unpack_kernel<ZsHasher>, ZS_WARPS * 32, smem) != cudaSuccess ||
+            cudaFuncSetAttribute(zstd_unpack_kernel<ZsPartialHasher>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess ||
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm_part, zstd_unpack_kernel<ZsPartialHasher>, ZS_WARPS * 32, smem) != cudaSuccess ||
+            per_sm < 1 || per_sm_part < 1) {
             g_last_error = std::string("zstd kernel setup failed: ") + cudaGetErrorString(cudaGetLastError());
             return nullptr;
         }
         ctx->zs_grid = ctx->sm_count * per_sm;
+        ctx->zs_grid_part = ctx->sm_count * per_sm_part;
     }
     if (cudaFuncSetAttribute(lz4_pack_blocks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P2_SMEM) != cudaSuccess ||
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->p2_per_sm, lz4_pack_blocks_kernel, 32 * P2_WARPS, P2_SMEM) != cudaSuccess ||
@@ -356,12 +360,19 @@ static cudaError_t launch_general(zpb_ctx *ctx, cudaStream_t s, const u8 *arch, 
     }
 }
 
-// zstd entries queued by the scan / general kernel: count at CNT_ZSTD, work counter at CNT_ZSTD_WORK
+// zstd entries queued by the scan / general kernel: count at CNT_ZSTD, work counter at CNT_ZSTD_WORK.  While
+// zpb_unpack_blocks_device drives the pipeline they are the frames of one entry, which leave stripe sums, not digests.
 static cudaError_t launch_zstd(zpb_ctx *ctx, cudaStream_t s, const u8 *arch, u8 *out, const zpb_entry *d_e,
                                int *d_status, u64 *d_digest) {
     u32 *cnt = (u32 *)ctx->d_counter.p;
-    zstd_unpack_kernel<<<ctx->zs_grid, ZS_WARPS * 32, ZS_WARPS * sizeof(ZstdShared), s>>>(
-        arch, out, d_e, (const u32 *)ctx->d_zlist.p, cnt + CNT_ZSTD, cnt + CNT_ZSTD_WORK, (u8 *)ctx->d_zlit.p, d_status, d_digest);
+    if (ctx->cur_partials)
+        zstd_unpack_kernel<ZsPartialHasher><<<ctx->zs_grid_part, ZS_WARPS * 32, ZS_WARPS * sizeof(ZstdShared), s>>>(
+            arch, out, d_e, (const u32 *)ctx->d_zlist.p, cnt + CNT_ZSTD, cnt + CNT_ZSTD_WORK, (u8 *)ctx->d_zlit.p, d_status,
+            d_digest, ctx->cur_partials);
+    else
+        zstd_unpack_kernel<ZsHasher><<<ctx->zs_grid, ZS_WARPS * 32, ZS_WARPS * sizeof(ZstdShared), s>>>(
+            arch, out, d_e, (const u32 *)ctx->d_zlist.p, cnt + CNT_ZSTD, cnt + CNT_ZSTD_WORK, (u8 *)ctx->d_zlit.p, d_status,
+            d_digest, nullptr);
     return cudaGetLastError();
 }
 
@@ -399,7 +410,7 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         // the kernels store 16 bytes at a time into the slot (include/zpack_b200.h: dst_off is 16-byte aligned)
         if (e.comp_size != 0 && (((uintptr_t)d_out + e.dst_off) & 15u))
             return fail(ctx, ZPB_E_ARG, "entry output slot is not 16-byte aligned");
-        any_zstd |= e.method == ZPB_METHOD_ZSTD;
+        any_zstd |= e.method == ZPB_METHOD_ZSTD || (internal && e.method == ZPB_M_ZSTD_FRAME);
         u64 c = (e.method == ZPB_METHOD_NONE || e.comp_size >= e.uncomp_size) ? e.comp_size / 16 : e.comp_size;
         c >>= 9;  // 512-byte cost buckets, descending
         const u32 key = c > 1023 ? 0u : 1023u - (u32)c;
@@ -425,7 +436,7 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
     }
 
     if (any_zstd && (!ctx->d_zlist.ensure(n * 4) ||
-                     !ctx->d_zlit.ensure((size_t)ctx->zs_grid * ZS_WARPS * ZS_LIT_SCRATCH)))
+                     !ctx->d_zlit.ensure((size_t)std::max(ctx->zs_grid, ctx->zs_grid_part) * ZS_WARPS * ZS_LIT_SCRATCH)))
         return fail(ctx, ZPB_E_NOMEM, "zstd scratch allocation failed");
     ctx->zstd_ms = 0.f;
     u64 *d_digest = (u64 *)ctx->d_res.p;
@@ -476,7 +487,10 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         // 16 384 entries on the unsplit walks fill the GPU by themselves and the merge is only extra work (text-only:
         // 2.23 -> 2.95 ms).  ZPB_PARSE_SPLIT=0 / 1 forces either.
         const bool split = set.parse_split >= 0 ? set.parse_split != 0 : slots <= 40000;
-        if (split) {
+        // A run of zstd frames (zpb_unpack_blocks_device) has no LZ4 block and nothing for the general kernel: the scan
+        // queues every frame for K4, so parse, execute and general are not launched (their events are still recorded).
+        const bool lz4_work = !(internal && slots == 0);
+        if (lz4_work && split) {
             // The light list first (stored blocks, runs: parsed within microseconds), so that the execute kernel, which
             // starts with the parse kernels, finds entries it can work on while text and record blocks are being walked;
             // then the split walk; then the blocks the split walk gave back (appended to the light list).
@@ -494,7 +508,7 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
             lz4_fast_parse_kernel<<<ctx->sm_count, K1_THREADS, K1_THREADS * K1_ROW, sp>>>(
                 d_archive, archive_size, d_fb, d_plist, (u32)(slots + 1), cnt, cnt + CNT_PARSE_LAST_WORK, d_fdesc, 2u);
             ctx->launches += 2;
-        } else {
+        } else if (lz4_work) {
             lz4_fast_parse_kernel<<<ctx->sm_count * k1_ctas, K1_THREADS, K1_THREADS * K1_ROW, sp>>>(
                 d_archive, archive_size, d_fb, d_plist, (u32)(slots + 1), cnt, cnt + CNT_PARSE_WORK, d_fdesc, 1u);
         }
@@ -513,8 +527,10 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         const int early = overlap ? (set.early_ctas > 0 && set.early_ctas <= k2_ctas ? set.early_ctas : (k2_ctas > 1 ? k2_ctas - 1 : 1))
                                   : k2_ctas;
         u32 *d_defer = overlap ? (u32 *)ctx->d_defer.p : nullptr;
-        CK(ctx, exec(early, s, d_xord, (u32)n, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
-        if (overlap) {
+        if (lz4_work) CK(ctx, exec(early, s, d_xord, (u32)n, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
+        if (overlap && !lz4_work) {
+            CK(ctx, cudaStreamWaitEvent(s, ctx->ev_p1, 0));
+        } else if (overlap) {
             if (k2_ctas > early) {
                 CK(ctx, cudaStreamWaitEvent(ctx->stream_b, ctx->ev_p1, 0));
                 CK(ctx, exec(k2_ctas - early, ctx->stream_b, d_xord, (u32)n, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
@@ -531,9 +547,12 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         CK(ctx, cudaEventRecord(ctx->ev_x1, s));
         CK(ctx, cudaEventRecord(ctx->evs[2], s));
         CK(ctx, cudaEventRecord(ctx->evs[3], s));
-        CK(ctx, launch_general(ctx, s, d_archive, archive_size, d_out, d_e, d_glist, 0u, cnt + CNT_GENERAL,
-                               cnt + CNT_GENERAL_WORK, d_status, d_digest));
-        ctx->launches += 4;
+        if (lz4_work) {
+            CK(ctx, launch_general(ctx, s, d_archive, archive_size, d_out, d_e, d_glist, 0u, cnt + CNT_GENERAL,
+                                   cnt + CNT_GENERAL_WORK, d_status, d_digest));
+            ctx->launches += 3;
+        }
+        ctx->launches += 1;
     } else {
         CK(ctx, cudaEventRecord(ctx->evs[0], s));
         CK(ctx, launch_general(ctx, s, d_archive, archive_size, d_out, d_e, d_ord, (u32)n, nullptr, cnt + CNT_WORK,

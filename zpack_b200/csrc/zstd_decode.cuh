@@ -935,15 +935,56 @@ ZPB_DEVINL int zstd_decode_entry(const ZWarp &w, ZstdShared &S, u8 *scratch, con
 #include "../../include/zpack_b200.h"
 #define ZS_WARPS 2
 
+// The entry's XXH3-64, streamed as the output front advances; the verdict of zpack_read_file (:466-468).
 struct ZsHasher {
     Xxh3Stream<32> s;
+    static constexpr int kFailed = ZPB_ST_DECOMPRESS_FAILED;   // lib/zpack_read.c:384-388
+    ZPB_DEVINL void init(u8 *dst, const zpb_entry &e, u64 *, const ZWarp &w) { s.init(dst, e.uncomp_size, w.g); }
     ZPB_DEVINL void advance(u64 front, const ZWarp &w) { s.advance(front, w.g); }
+    ZPB_DEVINL int finish(const zpb_entry &e, u64, u64 &dg, const ZWarp &w) {
+        dg = s.finish(w.g);
+        return !(e.flags & ZPB_F_NO_VERIFY) && dg != e.hash ? ZPB_ST_HASH_MISMATCH : ZPB_ST_OK;
+    }
 };
 
+// One frame of a zstd entry decoded frame-parallel (zpb_unpack_blocks_device, pseudo-entry ZPB_M_ZSTD_FRAME): every
+// complete KiB leaves its 16-stripe sums (64 bytes) at partials + (e.reserved + k) * 8, the layout lz4_fast_exec_kernel
+// writes for LZ4 blocks; xxh3_chain_kernel runs the scramble chain over them.  No digest, and a frame that fails or
+// decodes to another size than its pseudo-entry's declines the shard.
+struct ZsPartialHasher {
+    Xxh3Stream<32> s;   // base, alignment and the KiB cursor; its accumulators are not used
+    u64 *part;
+    static constexpr int kFailed = ZPB_ST_NOT_AVAILABLE;
+    ZPB_DEVINL void init(u8 *dst, const zpb_entry &e, u64 *partials, const ZWarp &w) {
+        s.init(dst, e.uncomp_size, w.g);
+        s.full_blocks = e.uncomp_size >> 10;   // every complete KiB: the entry's tail is folded by the chain kernel
+        part = partials + e.reserved * 8;
+    }
+    ZPB_DEVINL void advance(u64 front, const ZWarp &w) {
+        if (!(s.next_block < s.full_blocks && ((s.next_block + 1) << 10) <= front)) return;
+        w.g.sync();
+        while (s.next_block < s.full_blocks && ((s.next_block + 1) << 10) <= front) {
+            u64 s0 = 0, s1 = 0;
+            s.stripes_sum(s0, s1, s.base + (s.next_block << 10), 16, w.g);
+            s.fold(s0, s1, w.g);
+            if (w.l < 4) *reinterpret_cast<ulonglong2 *>(part + s.next_block * 8 + 2 * w.l) = make_ulonglong2(s0, s1);
+            ++s.next_block;
+        }
+    }
+    ZPB_DEVINL int finish(const zpb_entry &e, u64 produced, u64 &dg, const ZWarp &w) {
+        dg = 0;
+        if (produced != e.uncomp_size) return kFailed;
+        advance(produced, w);
+        return ZPB_ST_OK;
+    }
+};
+
+// `partials` is used by ZsPartialHasher only.
+template <class Hasher>
 __global__ void __launch_bounds__(ZS_WARPS * 32, 7)
 zstd_unpack_kernel(const u8 *__restrict__ archive, u8 *__restrict__ out, const zpb_entry *__restrict__ entries,
                    const u32 *__restrict__ list, const u32 *__restrict__ n_ptr, u32 *counter, u8 *scratch,
-                   int *status, u64 *digest) {
+                   int *status, u64 *digest, u64 *partials) {
     extern __shared__ __align__(16) u8 zs_smem[];
     ZstdShared &S = reinterpret_cast<ZstdShared *>(zs_smem)[threadIdx.x >> 5];
     ZWarp w;
@@ -957,19 +998,16 @@ zstd_unpack_kernel(const u8 *__restrict__ archive, u8 *__restrict__ out, const z
         const u32 idx = list[slot];
         const zpb_entry e = entries[idx];
         u8 *dst = out + e.dst_off;
-        ZsHasher hs;
-        hs.s.init(dst, e.uncomp_size, w.g);
+        Hasher hs;
+        hs.init(dst, e, partials, w);
 #ifdef ZPB_ZS_PROFILE
         w.t_last = clock64();
 #endif
         u64 produced = 0;
         int rc = zstd_decode_entry(w, S, lit_buf, archive + e.src_off, e.comp_size, dst, e.dst_cap, hs, &produced);
-        int st = rc ? ZPB_ST_DECOMPRESS_FAILED : ZPB_ST_OK;  // lib/zpack_read.c:384-388
+        int st = rc ? Hasher::kFailed : ZPB_ST_OK;
         u64 dg = 0;
-        if (st == ZPB_ST_OK) {
-            dg = hs.s.finish(w.g);  // :466
-            if (!(e.flags & ZPB_F_NO_VERIFY) && dg != e.hash) st = ZPB_ST_HASH_MISMATCH;
-        }
+        if (st == ZPB_ST_OK) st = hs.finish(e, produced, dg, w);
         if (w.l == 0) {
             status[idx] = st;
             digest[idx] = dg;

@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <algorithm>
 #include <atomic>
 #include <mutex>
 #include <new>
@@ -154,6 +155,28 @@ StreamState *state_of(zpack_stream *s) { return (StreamState *)s->xxh3_state; }
 
 bool known_method(int m) { return m == ZPACK_COMPRESSION_NONE || m == ZPACK_COMPRESSION_ZSTD || m == ZPACK_COMPRESSION_LZ4; }
 
+// Bytes of an entry's start that zstd_framed_head looks at
+constexpr size_t ZSTD_HEAD_BYTES = 7;
+
+// Whether a zstd entry starts the way this library's writer starts one of 64 KB frames: a single-segment frame of at
+// most 64 KB, no checksum, no dictionary.  Anything else — the reference's one frame of dependent blocks, this
+// library's frames from before the 64 KB layout — has nothing for the frame-parallel path.
+bool zstd_framed_head(const zpack_u8 *p, size_t n) {
+    if (n < 6 || get32(p) != 0xFD2FB528u) return false;
+    const unsigned fhd = p[4];
+    if (!(fhd & 0x20) || (fhd & 0x0F)) return false;
+    if ((fhd >> 6) == 0) return true;                                  // 1-byte Frame_Content_Size
+    return (fhd >> 6) == 1 && n >= 7 && get16(p + 5) + 256u <= 65536u;  // 2 bytes, holding size - 256
+}
+
+// Entries gpu_unpack_one first offers to zpb_unpack_entry_blocks_host (`head`: the first bytes of the entry, n of
+// them).  zstd is routed on decoded size: a highly compressible file can be small on disk, and one warp's decode time
+// grows with the bytes it writes.
+bool block_path_entry(const zpack_file_entry &e, const zpack_u8 *head, size_t n) {
+    return (e.comp_method == ZPACK_COMPRESSION_LZ4 && e.comp_size >= ZPB_ZSTD_FRAMED_MIN) ||
+           (e.comp_method == ZPACK_COMPRESSION_ZSTD && e.uncomp_size >= ZPB_ZSTD_FRAMED_MIN && zstd_framed_head(head, n));
+}
+
 // One entry through the GPU: compressed bytes `comp` -> dst[0..max_size).  Returns an enum zpack_result.
 int gpu_unpack_one(const zpack_u8 *comp, zpack_u64 comp_size, zpack_u8 *dst, size_t max_size, const zpack_file_entry *e,
                    size_t *last_return) {
@@ -165,9 +188,10 @@ int gpu_unpack_one(const zpack_u8 *comp, zpack_u64 comp_size, zpack_u8 *dst, siz
     d.uncomp_size = e->uncomp_size; d.hash = e->hash; d.method = e->comp_method;
     int32_t st = 0;
     uint64_t dg = 0;
-    // a large LZ4 entry written with independent blocks (what this library's writer emits) is decoded block-parallel,
-    // chunks pipelined over PCIe; anything else — and anything that path declines — is one dependency chain
-    if (e->comp_method == ZPACK_COMPRESSION_LZ4 && comp_size >= (4u << 20)) {
+    // a large LZ4 entry written with independent blocks, or a large zstd entry written as 64 KB frames (what this
+    // library's writer emits), is decoded block-parallel, chunks pipelined over PCIe; anything else — and anything that
+    // path declines — is one dependency chain
+    if (block_path_entry(*e, comp, (size_t)std::min<zpack_u64>(comp_size, ZSTD_HEAD_BYTES))) {
         int rc = zpb_unpack_entry_blocks_host(g, comp, comp_size, dst, max_size, e->uncomp_size, e->hash, 0, &st, &dg);
         if (rc == ZPB_OK) {
             if (last_return) *last_return = (size_t)st;
@@ -363,8 +387,16 @@ bool same_fields(const zpack_file_entry &a, const zpack_file_entry &b) {
            a.comp_method == b.comp_method;
 }
 bool plain_entry(const zpack_reader *r, const zpack_file_entry &e) {      // what zpack_read_file would hand to the GPU as one chain
-    return e.comp_size && e.offset < r->file_size && e.comp_size < r->file_size - e.offset && known_method(e.comp_method) &&
-           !(e.comp_method == ZPACK_COMPRESSION_LZ4 && e.comp_size >= (4u << 20));
+    if (!e.comp_size || e.offset >= r->file_size || e.comp_size >= r->file_size - e.offset || !known_method(e.comp_method))
+        return false;
+    if (e.comp_method != ZPACK_COMPRESSION_ZSTD || e.uncomp_size < ZPB_ZSTD_FRAMED_MIN) return !block_path_entry(e, nullptr, 0);
+    // a large zstd entry leaves the read-ahead batch only when it is 64 KB frames: its first bytes say so
+    zpack_u8 head[ZSTD_HEAD_BYTES];
+    const size_t n = (size_t)std::min<zpack_u64>(e.comp_size, sizeof head);
+    int err;
+    if (r->buffer) memcpy(head, r->buffer + e.offset, n);
+    else if (!r->file || !read_at(r->file, e.offset, head, n, &err)) return true;   // the read that follows reports it
+    return !block_path_entry(e, head, n);
 }
 // Decodes entries [idx, idx + k) into the cache; false = nothing cached (the caller takes the one-entry path).
 bool readahead_fill(zpack_reader *r, zpack_u64 idx) {

@@ -44,7 +44,10 @@ File = np.dtype(
 #: numpy dtype of `struct zpb_block` (16 bytes)
 Block = np.dtype([("src_off", "<u8"), ("comp_size", "<u4"), ("flags", "<u4")])
 BLK_STORED = 1
+BLK_ZSTD = 2
 INDEX_UNSUPPORTED = 1
+#: ZPB_ZSTD_FRAMED_MIN: zstd files of at least this many bytes are written as one frame per 64 KB (zstd_frame_index)
+ZSTD_FRAMED_MIN = 4 << 20
 #: numpy dtype of `struct zpb_arc_entry` (64 bytes): one row of a device-resident archive's directory
 ArcEntry = np.dtype(
     [("src_off", "<u8"), ("comp_size", "<u8"), ("uncomp_size", "<u8"), ("hash", "<u8"), ("name_off", "<u8"),
@@ -57,7 +60,7 @@ EXPORTS = [
     "zpb_launch_count", "zpb_unpack_device", "zpb_unpack_host", "zpb_xxh3_device", "zpb_xxh3_host",
     "zpb_pack_bound", "zpb_pack_device", "zpb_pack_host", "zpb_last_kernel_ms", "zpb_last_pack_stage_ms", "zpb_set_tuning",
     "zpb_last_stage_ms", "zpb_set_fast_path", "zpb_set_overlap", "zpb_set_lz4hc", "zpb_set_zstd_entropy", "zpb_last_zstd_ms",
-    "zpb_lz4_frame_index", "zpb_unpack_blocks_device", "zpb_blocks_digest", "zpb_last_chain_ms",
+    "zpb_lz4_frame_index", "zpb_zstd_frame_index", "zpb_unpack_blocks_device", "zpb_blocks_digest", "zpb_last_chain_ms",
     "zpb_unpack_entry_blocks_host", "zpb_device_count",
     "zpb_archive_open_device", "zpb_archive_build_device", "zpb_copy_entries_device", "zpb_last_archive_ms",
     "zpb_file_read_device", "zpb_file_write_device",
@@ -107,6 +110,7 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.zpb_set_zstd_entropy.argtypes = [vp, C.c_int]
     lib.zpb_last_zstd_ms.argtypes = [vp, C.POINTER(C.c_float)]
     lib.zpb_lz4_frame_index.argtypes = [vp, u64, u64, vp, u64, u64p, C.POINTER(C.c_uint32), u64p]
+    lib.zpb_zstd_frame_index.argtypes = [vp, u64, u64, vp, u64, u64p, u64p]
     lib.zpb_unpack_blocks_device.argtypes = [vp, vp, u64, vp, u64, vp, u64, C.c_uint32, u64, i32p, vp]
     lib.zpb_blocks_digest.argtypes = [vp, vp, vp, u64, u64, vp, u64p, vp]
     lib.zpb_last_chain_ms.argtypes = [vp, C.POINTER(C.c_float)]
@@ -228,6 +232,24 @@ def lz4_frame_index(frame: np.ndarray, archive_off: int = 0):
     return blocks[:n.value].copy(), bs.value, (None if cs.value == 2**64 - 1 else cs.value)
 
 
+def zstd_frame_index(entry: np.ndarray, archive_off: int = 0):
+    """Host-side framing walk of a zstd entry written as 64 KB frames (no GPU needed, no codec work): returns
+    (frames: Block[n] with flags BLK_ZSTD, content_size), or None when the entry does not have that shape
+    (zpb_zstd_frame_index -> ZPB_INDEX_UNSUPPORTED)."""
+    lib = load_library()
+    entry = np.ascontiguousarray(entry, np.uint8)
+    n, cs = C.c_uint64(), C.c_uint64()
+    cap = len(entry) // 9 + 1   # every frame costs at least a 6-byte header + a 3-byte block header
+    frames = np.zeros(cap, Block)
+    rc = lib.zpb_zstd_frame_index(entry.ctypes.data, len(entry), archive_off, frames.ctypes.data, cap,
+                                  C.byref(n), C.byref(cs))
+    if rc == INDEX_UNSUPPORTED:
+        return None
+    if rc != 0:
+        raise ZpbError(f"zpb_zstd_frame_index: {rc}")
+    return frames[:n.value].copy(), cs.value
+
+
 class Context:
     """One GPU context (`zpb_ctx`): scratch arenas, a stream, CUDA-event timers."""
 
@@ -319,7 +341,8 @@ class Context:
     # ---- one large entry, sharded by blocks (C5) ------------------------------------------------
     def unpack_blocks_device(self, d_archive, archive_size: int, d_out, out_size: int, blocks: np.ndarray,
                              block_size: int, shard_uncomp_size: int, stream: int = 0) -> int:
-        """Decode a contiguous run of one entry's independent blocks; returns the shard status."""
+        """Decode a contiguous run of one entry's independent blocks (LZ4) or frames (zstd, flags BLK_ZSTD; block_size
+        65536); returns the shard status."""
         assert blocks.dtype == Block and blocks.flags.c_contiguous
         st = C.c_int32(-1)
         self._check(self.lib.zpb_unpack_blocks_device(self.h, _ptr(d_archive), archive_size, _ptr(d_out), out_size,
@@ -343,8 +366,9 @@ class Context:
 
     def unpack_entry_blocks_host(self, h_entry, comp_size: int, h_out, out_cap: int, uncomp_size: int,
                                  expect_hash: int, flags: int = 0):
-        """One large block-independent LZ4 entry, host buffers (pipelined chunks + XXH3 relay).
-        Returns (status, digest), or None when the entry is not eligible for the block path."""
+        """One large block-independent LZ4 entry, or one zstd entry of 64 KB frames (what pack_* writes from
+        ZSTD_FRAMED_MIN on), host buffers (pipelined chunks + XXH3 relay).  The index is chosen by the entry's magic
+        number.  Returns (status, digest), or None when the entry is not eligible for the block path."""
         st, dg = C.c_int32(-1), C.c_uint64(0)
         rc = self.lib.zpb_unpack_entry_blocks_host(self.h, _ptr(h_entry), comp_size, _ptr(h_out), out_cap,
                                                    uncomp_size, expect_hash, flags, C.byref(st), C.byref(dg))
