@@ -96,7 +96,12 @@ uint64_t    zpb_launch_count(const zpb_ctx *ctx);
 /* unpack + verify ------------------------------------------------------------------------- */
 /* Device-resident batch.  d_archive/d_out are device pointers; entries/status/digest are HOST
  * arrays of n elements (descriptor upload and result download are part of the call).
- * `stream` is a cudaStream_t (NULL = the context's own stream).  Synchronous on return. */
+ * `stream` is a cudaStream_t (NULL = the context's own stream).  Synchronous on return.
+ * An entry of at least ZPB_ZSTD_FRAMED_MIN decoded bytes that is an LZ4 frame of independent 64 KB blocks, or a zstd
+ * entry of 64 KB frames (what zpb_pack_* writes; the shapes zpb_lz4_frame_index / zpb_zstd_frame_index accept), is
+ * decoded block-parallel inside the batch: its framing is indexed on the device and each 64 KB becomes a row of its
+ * own, so one large entry costs about what the block path costs for it alone.  Other large entries (linked blocks,
+ * one zstd frame) are decoded by one warp.  Statuses and digests are the same either way. */
 int zpb_unpack_device(zpb_ctx *ctx, const uint8_t *d_archive, uint64_t archive_size,
                       uint8_t *d_out, uint64_t out_size, const zpb_entry *entries, uint64_t n,
                       int32_t *status, uint64_t *digest, void *stream);
@@ -104,7 +109,8 @@ int zpb_unpack_device(zpb_ctx *ctx, const uint8_t *d_archive, uint64_t archive_s
 /* Same with host buffers: copies [lo,hi) of the archive that the entries touch to the device,
  * unpacks, copies each entry's uncomp_size bytes back into h_out + dst_off.  Batches of more than a few
  * hundred MB are pipelined in chunks over several streams (H2D, kernels and D2H of different chunks
- * overlap); pinned host buffers are needed for the copies to be asynchronous. */
+ * overlap); pinned host buffers are needed for the copies to be asynchronous.  Large entries are decoded
+ * block-parallel as in zpb_unpack_device; an entry stays whole inside one chunk. */
 int zpb_unpack_host(zpb_ctx *ctx, const uint8_t *h_archive, uint64_t archive_size,
                     uint8_t *h_out, uint64_t out_size, const zpb_entry *entries, uint64_t n,
                     int32_t *status, uint64_t *digest);

@@ -29,6 +29,7 @@ enum CounterSlot : u32 {
     CNT_GENERAL_WORK = 4,      // work counter of the general kernel over the fast path's list
     CNT_ZSTD = 5,              // length of the zstd list
     CNT_ZSTD_WORK = 6,         // work counter of zstd_unpack_kernel
+    CNT_ZSTD_FRAMES = 7,       // length of the list of 64 KB zstd frames (pseudo-rows), and CNT_ZSTD_FRAMES_WORK
     CNT_PARSE_HEAVY = 8,       // lengths of the parse lists by weight: heavy, medium (+1), light (+2)
     CNT_PARSE_MEDIUM = 9,
     CNT_PARSE_LIGHT = 10,
@@ -37,6 +38,7 @@ enum CounterSlot : u32 {
     CNT_PARSE_WORK = 13,       // work counter of the first unsplit parse launch
     CNT_SPLIT_GIVEN_BACK = 14, // statistics: blocks the split walk gave back to the unsplit walk
     CNT_SPLIT_RETRIES = 15,    // statistics: second attempts of the split walk
+    CNT_ZSTD_FRAMES_WORK = 16, // work counter of zstd_unpack_kernel over the frame list
     CNT_LIGHT_FIRST = 17,      // light-list length the first parse launch walked (the last launch walks the rest)
     CNT_PARSE_LAST_WORK = 18,  // work counter of the last parse launch
     CNT_PACK_BLOCKS_WORK = 32, // work counter of lz4_pack_blocks_kernel

@@ -62,6 +62,7 @@ static_assert((FAST_RING & FAST_RMASK) == 0 && FAST_RING % 1024u == 0, "output r
 #define FE_FAST    1u   // block table filled, goes through K1/K2
 #define FE_GENERAL 2u   // handed to the general kernel
 #define FE_ZSTD    3u   // handed to the zstd kernel (zstd_decode.cuh)
+#define FE_SPLIT   4u   // decoded by its pseudo-rows (split_entries.cuh)
 
 #define FAST_DESC_PER_BLOCK 2060ull
 #define K1_HEAVY   (24u << 10)   // compressed block bytes: heavy / medium / light parse work lists
@@ -79,6 +80,9 @@ static_assert((FAST_RING & FAST_RMASK) == 0 && FAST_RING % 1024u == 0, "output r
 // Likewise one whole zstd frame of an entry written as 64 KB frames (zpb_zstd_frame_index): queued for the zstd kernel,
 // whose ZsPartialHasher instantiation leaves the frame's stripe sums at `reserved` the same way.
 #define ZPB_M_ZSTD_FRAME  0x103u
+// A large entry of a batch that split_index_kernel (split_entries.cuh) has cut into such rows: the scan kernel leaves it
+// alone, and xxh3_chain_batch_kernel writes its status and digest.
+#define ZPB_M_SPLIT       0x104u
 #define ZPB_F_STORED_BLK  0x100u
 #define FE_LINK_NONE    0u
 #define FE_LINK_WINDOW  1u   // blocks of the frame share the 64 KB window (B.Indep = 0)
@@ -212,6 +216,8 @@ lz4_fast_scan_kernel(const u8 *__restrict__ archive, u64 asz, const zpb_entry *_
         }
     } else if (e.method == ZPB_METHOD_ZSTD || e.method == ZPB_M_ZSTD_FRAME) {
         f.state = FE_ZSTD;                                     // guards passed: the zstd kernel decodes it
+    } else if (e.method == ZPB_M_SPLIT) {
+        f.state = FE_SPLIT;
     } else {
         f.state = FE_GENERAL;                                  // unknown method: the general kernel answers
     }
@@ -221,8 +227,10 @@ lz4_fast_scan_kernel(const u8 *__restrict__ archive, u64 asz, const zpb_entry *_
     } else if (f.state == FE_GENERAL) {
         general_list[atomicAdd(&counters[CNT_GENERAL], 1u)] = idx;
     } else if (f.state == FE_ZSTD) {
-        zstd_list[atomicAdd(&counters[CNT_ZSTD], 1u)] = idx;
-    } else {
+        // frames leave stripe sums (zstd_unpack_kernel<ZsPartialHasher>): their own list, at zstd_list + n
+        if (e.method == ZPB_M_ZSTD_FRAME) zstd_list[n + atomicAdd(&counters[CNT_ZSTD_FRAMES], 1u)] = idx;
+        else zstd_list[atomicAdd(&counters[CNT_ZSTD], 1u)] = idx;
+    } else if (f.state == FE_FAST) {
         for (u32 b = 0; b < f.nblocks; ++b)
             if (!(fb[a.slot_base + b].flags & FB_STORED))
             {

@@ -18,15 +18,15 @@
 #define XC_BATCH  64u   // KiB steps per batch: 64 x 64 B = 4 KiB of shared memory
 #define XC_STAGES 8u    // batches in flight (cp.async ring, 32 KiB)
 
+// The chain of one warp (all 32 lanes), shared by xxh3_chain_kernel and xxh3_chain_batch_kernel (split_entries.cuh).
 // acc[8] in xxHash order.  nscr = how many leading S_n are followed by a scramble (all of the shard's
 // complete KiBs, except that the entry's very last KiB is never scrambled: it belongs to the tail).
 // When `final`: tail_ptr = decoded bytes starting at entry position tail_pos (<= both the tail start
-// and total - 64), total = the entry's uncomp_size.
-__global__ void __launch_bounds__(32)
-xxh3_chain_kernel(const u64 *__restrict__ partials, u64 nscr, const u64 *__restrict__ acc_in, u64 *acc_out,
-                  int final, const u8 *tail_ptr, u64 tail_pos, u64 total, u64 *digest_out) {
-    __shared__ ulonglong2 stage[XC_STAGES][XC_BATCH * 4];
-    const int lane = threadIdx.x;
+// and total - 64), total = the entry's uncomp_size; returns the digest (0 when not final).
+ZPB_DEVINL u64 xxh3_chain_body(ulonglong2 (*stage)[XC_BATCH * 4], const u64 *__restrict__ partials, u64 nscr,
+                               const u64 *__restrict__ acc_in, u64 *acc_out, int final, const u8 *tail_ptr, u64 tail_pos,
+                               u64 total) {
+    const int lane = threadIdx.x & 31;
     const int j = lane & 3;
     const int i8 = lane & 7;      // the chain runs one accumulator per lane on lanes 0-7: every instruction of a
                                   // step then serves all 8 chains (a warp instruction costs the same for 1 or 32 lanes)
@@ -105,7 +105,7 @@ xxh3_chain_kernel(const u64 *__restrict__ partials, u64 nscr, const u64 *__restr
         __syncwarp();
     }
     if (acc_out && lane < 8) acc_out[i8] = a;
-    if (!final) return;
+    if (!final) return 0;
 
     // ---- tail (xxhash.h:3701-3711) + merge (:3714-3747): pairwise layout again (lane l works for pair l & 3)
     const u64 a0 = __shfl_sync(0xffffffffu, a, 2 * j);
@@ -139,5 +139,13 @@ xxh3_chain_kernel(const u64 *__restrict__ partials, u64 nscr, const u64 *__restr
         m += __shfl_xor_sync(0xffffffffu, m, 2);
         dg = xxh3_avalanche(total * XXH_P64_1 + m);
     }
-    if (lane == 0 && digest_out) *digest_out = dg;
+    return dg;
+}
+
+__global__ void __launch_bounds__(32)
+xxh3_chain_kernel(const u64 *__restrict__ partials, u64 nscr, const u64 *__restrict__ acc_in, u64 *acc_out,
+                  int final, const u8 *tail_ptr, u64 tail_pos, u64 total, u64 *digest_out) {
+    __shared__ ulonglong2 stage[XC_STAGES][XC_BATCH * 4];
+    const u64 dg = xxh3_chain_body(stage, partials, nscr, acc_in, acc_out, final, tail_ptr, tail_pos, total);
+    if (final && threadIdx.x == 0 && digest_out) *digest_out = dg;
 }

@@ -18,6 +18,7 @@
 #include "pack_kernel.cuh"
 #include "zstd_decode.cuh"
 #include "xxh3_chain.cuh"
+#include "split_entries.cuh"
 #include "archive_kernels.cuh"
 
 static thread_local std::string g_last_error = "";
@@ -157,6 +158,10 @@ struct zpb_ctx {
     u64 *cur_partials = nullptr;       // non-null only while zpb_unpack_blocks_device drives the pipeline
     u64 blk_uncomp = 0;                // decoded bytes of the last shard (0 = none / declined)
     float chain_ms = 0.f;
+    // large entries of a batch decoded block-parallel (split_entries.cuh): candidates, their stripe sums
+    std::vector<SplitJob> h_jobs;
+    DevBuf d_jobs, d_bpart;
+    bool no_split = false;             // set during the unsplit pass over the entries whose pseudo-rows did not all decode
     // device-resident container operations (archive_api.inl): entry table, record offsets, chunk table, totals, names; CDR walk tables
     DevBuf d_arc_e, d_arc_rec, d_arc_chunk, d_arc_work, d_arc_scan, d_arc_tot, d_arc_names, d_cdr_jump, d_cdr_cnt, d_cdr_j2, d_cdr_anchor;
     float arc_ms[3] = {0, 0, 0};       // layout + directory kernels, copy kernel, open kernels of the last call
@@ -249,6 +254,10 @@ extern "C" zpb_ctx *zpb_create(int device) {
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctx->pk_per_sm, lz4_pack_kernel, 32 * PK_WARPS, 0) != cudaSuccess ||
         ctx->p2_per_sm < 1 || ctx->pk_per_sm < 1) {
         g_last_error = std::string("pack kernel setup failed: ") + cudaGetErrorString(cudaGetLastError());
+        return nullptr;
+    }
+    if (cudaFuncSetAttribute(split_index_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SPLIT_SMEM) != cudaSuccess) {
+        g_last_error = std::string("split kernel setup failed: ") + cudaGetErrorString(cudaGetLastError());
         return nullptr;
     }
     if (cudaFuncSetAttribute(lz4hc_match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HC_SMEM) != cudaSuccess) {
@@ -360,15 +369,16 @@ static cudaError_t launch_general(zpb_ctx *ctx, cudaStream_t s, const u8 *arch, 
     }
 }
 
-// zstd entries queued by the scan / general kernel: count at CNT_ZSTD, work counter at CNT_ZSTD_WORK.  While
-// zpb_unpack_blocks_device drives the pipeline they are the frames of one entry, which leave stripe sums, not digests.
+// zstd entries queued by the scan / general kernel: count at CNT_ZSTD, work counter at CNT_ZSTD_WORK.  64 KB frames
+// (pseudo-rows of zpb_unpack_blocks_device or of a split entry) are queued at zlist + n_rows, count at CNT_ZSTD_FRAMES:
+// they leave stripe sums at `partials`, not digests.
 static cudaError_t launch_zstd(zpb_ctx *ctx, cudaStream_t s, const u8 *arch, u8 *out, const zpb_entry *d_e,
-                               int *d_status, u64 *d_digest) {
+                               int *d_status, u64 *d_digest, bool frames, u64 n_rows, u64 *partials) {
     u32 *cnt = (u32 *)ctx->d_counter.p;
-    if (ctx->cur_partials)
+    if (frames)
         zstd_unpack_kernel<ZsPartialHasher><<<ctx->zs_grid_part, ZS_WARPS * 32, ZS_WARPS * sizeof(ZstdShared), s>>>(
-            arch, out, d_e, (const u32 *)ctx->d_zlist.p, cnt + CNT_ZSTD, cnt + CNT_ZSTD_WORK, (u8 *)ctx->d_zlit.p, d_status,
-            d_digest, ctx->cur_partials);
+            arch, out, d_e, (const u32 *)ctx->d_zlist.p + n_rows, cnt + CNT_ZSTD_FRAMES, cnt + CNT_ZSTD_FRAMES_WORK,
+            (u8 *)ctx->d_zlit.p, d_status, d_digest, partials);
     else
         zstd_unpack_kernel<ZsHasher><<<ctx->zs_grid, ZS_WARPS * 32, ZS_WARPS * sizeof(ZstdShared), s>>>(
             arch, out, d_e, (const u32 *)ctx->d_zlist.p, cnt + CNT_ZSTD, cnt + CNT_ZSTD_WORK, (u8 *)ctx->d_zlit.p, d_status,
@@ -376,16 +386,44 @@ static cudaError_t launch_zstd(zpb_ctx *ctx, cudaStream_t s, const u8 *arch, u8 
     return cudaGetLastError();
 }
 
+// A row the batch decodes block-parallel when split_index_kernel accepts its framing: LZ4 or zstd, at least
+// ZPB_ZSTD_FRAMED_MIN decoded bytes, and past the scan kernel's guards (those rows get their verdict there).
+static bool split_candidate(const zpb_entry &e, u64 archive_size) {
+    return (e.method == ZPB_METHOD_LZ4 || e.method == ZPB_METHOD_ZSTD) && e.uncomp_size >= ZPB_ZSTD_FRAMED_MIN &&
+           e.comp_size != 0 && e.dst_cap >= e.uncomp_size && e.src_off <= archive_size &&
+           e.comp_size <= archive_size - e.src_off;
+}
+
 static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_size, u8 *d_out,
                               u64 out_size, const zpb_entry *entries, u64 n, int32_t *status,
                               u64 *digest, cudaStream_t s) {
     if (n == 0) return ZPB_OK;
     if (n > 0x7fffffffull) return fail(ctx, ZPB_E_ARG, "too many entries in one batch");
-    size_t desc_b = n * sizeof(zpb_entry), ord_b = n * sizeof(u32);
-    size_t res_b = n * (sizeof(int) + sizeof(u64));
+    const bool internal = ctx->cur_partials != nullptr;   // method codes above a byte are internal (comp_method is a u8, lib/zpack.h:79)
+    // Large entries (split_entries.cuh): one job per candidate, its pseudo-rows after the caller's n rows.  The rows stay
+    // inert (comp_size 0) unless the pre-pass accepts the entry's framing.
+    std::vector<SplitJob> &jobs = ctx->h_jobs;
+    jobs.clear();
+    u64 N = n, kibs = 0;
+    if (!internal && !ctx->no_split && ctx->set.fast)
+        for (u64 i = 0; i < n; ++i)
+            if (split_candidate(entries[i], archive_size)) {
+                SplitJob j;
+                j.parent = (u32)i;
+                j.row0 = (u32)N;
+                j.nrows = (u32)((entries[i].uncomp_size + 65535) >> 16);
+                j.kib0 = kibs;
+                j.desc_base = 0; j.slot_base = 0;
+                N += j.nrows;
+                kibs += (entries[i].uncomp_size + 1023) >> 10;
+                jobs.push_back(j);
+            }
+    if (N > 0x7fffffffull) return fail(ctx, ZPB_E_ARG, "too many entries in one batch");
+    size_t desc_b = N * sizeof(zpb_entry), ord_b = N * sizeof(u32);
+    size_t res_b = N * (sizeof(int) + sizeof(u64));
     if (!ctx->d_desc.ensure(desc_b) || !ctx->d_order.ensure(ord_b) || !ctx->d_res.ensure(res_b + 64) ||
         !ctx->d_counter.ensure(CNT_SLOTS * sizeof(u32)) || !ctx->d_order2.ensure(ord_b) || !ctx->d_defer.ensure(ord_b) ||
-        !ctx->h_stage.ensure(desc_b + 2 * ord_b + res_b + 64 + n * sizeof(FastAux)))
+        !ctx->h_stage.ensure(desc_b + 2 * ord_b + res_b + 64 + N * sizeof(FastAux)))
         return fail(ctx, ZPB_E_NOMEM, "scratch allocation failed");
 
     // ---- one pass over the descriptors (the GPU idles while the host prepares a batch, so this is kept to a single
@@ -396,13 +434,13 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
     zpb_entry *h_desc = (zpb_entry *)hs;
     u32 *h_order = (u32 *)(hs + desc_b);
     FastAux *h_aux = (FastAux *)(hs + desc_b + ord_b + res_b + 64);
-    ctx->h_keys.resize(n);
+    ctx->h_keys.resize(N);
     u16 *keys = ctx->h_keys.data();
     u32 head[1025];
     memset(head, 0, sizeof(head));
-    bool any_zstd = false;
-    const bool internal = ctx->cur_partials != nullptr;   // method codes above a byte are internal (comp_method is a u8, lib/zpack.h:79)
+    bool any_zstd = false, any_frames = false;
     u64 slots = 0, ndesc = 0;
+    size_t jn = 0;
     for (u64 i = 0; i < n; ++i) {
         zpb_entry e = entries[i];
         if (e.comp_size != 0 && (e.dst_off > out_size || e.dst_cap > out_size - e.dst_off))
@@ -410,40 +448,70 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         // the kernels store 16 bytes at a time into the slot (include/zpack_b200.h: dst_off is 16-byte aligned)
         if (e.comp_size != 0 && (((uintptr_t)d_out + e.dst_off) & 15u))
             return fail(ctx, ZPB_E_ARG, "entry output slot is not 16-byte aligned");
-        any_zstd |= e.method == ZPB_METHOD_ZSTD || (internal && e.method == ZPB_M_ZSTD_FRAME);
+        any_zstd |= e.method == ZPB_METHOD_ZSTD;
+        any_frames |= internal && e.method == ZPB_M_ZSTD_FRAME;
         u64 c = (e.method == ZPB_METHOD_NONE || e.comp_size >= e.uncomp_size) ? e.comp_size / 16 : e.comp_size;
         c >>= 9;  // 512-byte cost buckets, descending
         const u32 key = c > 1023 ? 0u : 1023u - (u32)c;
         keys[i] = (u16)key;
         ++head[key + 1];
         h_aux[i] = fast_entry_layout(e, slots, ndesc);
+        if (jn < jobs.size() && jobs[jn].parent == i) {
+            SplitJob &j = jobs[jn++];
+            any_frames |= e.method == ZPB_METHOD_ZSTD;
+            if (e.method == ZPB_METHOD_LZ4) {
+                // the blocks' FastBlock slots and descriptors: the parent's own (fast_scan_lz4's layout), or for 2 GiB
+                // and more, where the parent gets none, the same amount reserved here
+                if (h_aux[i].nslots == 0) {
+                    h_aux[i].slot_base = (u32)slots; h_aux[i].desc_base = ndesc;
+                    slots += j.nrows + 2;
+                    ndesc += ((e.comp_size / 3 + FAST_DESC_PER_BLOCK * (j.nrows + 2) + 8) + 3) & ~3ull;
+                }
+                j.slot_base = h_aux[i].slot_base;
+                j.desc_base = h_aux[i].desc_base;
+            }
+            // the pseudo-rows: inert until the pre-pass fills them, ordered by the parent's compressed bytes per block
+            u64 cb = (e.comp_size / j.nrows) >> 9;
+            const u32 pkey = cb > 1023 ? 0u : 1023u - (u32)cb;
+            memset(h_desc + j.row0, 0, (size_t)j.nrows * sizeof(zpb_entry));
+            memset(h_aux + j.row0, 0, (size_t)j.nrows * sizeof(FastAux));
+            for (u32 k = 0; k < j.nrows; ++k) keys[j.row0 + k] = (u16)pkey;
+            head[pkey + 1] += j.nrows;
+        }
         if (!internal && e.method > 0xFFu) e.method = 0xFFu;
         h_desc[i] = e;
     }
     if (slots > 0x7fffffffull) return fail(ctx, ZPB_E_ARG, "too many blocks in one batch");
     for (u32 k = 0; k < 1024; ++k) head[k + 1] += head[k];
-    for (u64 i = 0; i < n; ++i) h_order[head[keys[i]]++] = (u32)i;   // counting sort: O(n), stable
+    for (u64 i = 0; i < N; ++i) h_order[head[keys[i]]++] = (u32)i;   // counting sort: O(n), stable
     // The execute kernel starts while the heaviest blocks are still being parsed, so ITS order leads with the
     // entries that are parsed (almost) at once — stored and highly compressible ones, the cheap end of the list —
     // and continues with the rest, expensive first as before.
-    u32 *h_order2 = (u32 *)(hs + desc_b + ord_b + res_b + 64 + n * sizeof(FastAux));
+    u32 *h_order2 = (u32 *)(hs + desc_b + ord_b + res_b + 64 + N * sizeof(FastAux));
     {
         u64 ncheap = 0;
         const u32 front_buckets = ctx->set.front_buckets;
-        while (ncheap < n && keys[h_order[n - 1 - ncheap]] >= 1024u - front_buckets) ++ncheap;   // cost below front_buckets x 512 B (default 16 KB)
-        for (u64 k = 0; k < ncheap; ++k) h_order2[k] = h_order[n - 1 - k];
-        for (u64 k = ncheap; k < n; ++k) h_order2[k] = h_order[k - ncheap];
+        while (ncheap < N && keys[h_order[N - 1 - ncheap]] >= 1024u - front_buckets) ++ncheap;   // cost below front_buckets x 512 B (default 16 KB)
+        for (u64 k = 0; k < ncheap; ++k) h_order2[k] = h_order[N - 1 - k];
+        for (u64 k = ncheap; k < N; ++k) h_order2[k] = h_order[k - ncheap];
     }
 
-    if (any_zstd && (!ctx->d_zlist.ensure(n * 4) ||
+    if ((any_zstd || any_frames) && (!ctx->d_zlist.ensure(N * 8) ||
                      !ctx->d_zlit.ensure((size_t)std::max(ctx->zs_grid, ctx->zs_grid_part) * ZS_WARPS * ZS_LIT_SCRATCH)))
         return fail(ctx, ZPB_E_NOMEM, "zstd scratch allocation failed");
     ctx->zstd_ms = 0.f;
     u64 *d_digest = (u64 *)ctx->d_res.p;
-    int *d_status = (int *)((u8 *)ctx->d_res.p + n * sizeof(u64));
+    int *d_status = (int *)((u8 *)ctx->d_res.p + N * sizeof(u64));
     const zpb_entry *d_e = (const zpb_entry *)ctx->d_desc.p;
     const u32 *d_ord = (const u32 *)ctx->d_order.p;
     u32 *cnt = (u32 *)ctx->d_counter.p;   // slots: CounterSlot (common.cuh)
+    u64 *d_part = ctx->cur_partials;      // stripe sums of 64 KB rows: the shard's, or the batch's split entries'
+    if (!jobs.empty()) {
+        if (!ctx->d_jobs.ensure(jobs.size() * sizeof(SplitJob)) || !ctx->d_bpart.ensure((kibs + 1) * 64))
+            return fail(ctx, ZPB_E_NOMEM, "split scratch allocation failed");
+        d_part = (u64 *)ctx->d_bpart.p;
+        CK(ctx, cudaMemcpyAsync(ctx->d_jobs.p, jobs.data(), jobs.size() * sizeof(SplitJob), cudaMemcpyHostToDevice, s));
+    }
 
     CK(ctx, cudaMemcpyAsync(ctx->d_desc.p, h_desc, desc_b, cudaMemcpyHostToDevice, s));
     CK(ctx, cudaMemcpyAsync(ctx->d_order.p, h_order, ord_b, cudaMemcpyHostToDevice, s));
@@ -451,18 +519,25 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
     const Settings &set = ctx->set;
     if (set.fast) {
         // ---- scan -> parse -> exec (lz4_fast.cuh), then the general kernel over whatever they declined
-        size_t aux_b = n * sizeof(FastAux);
-        if (!ctx->d_aux.ensure(aux_b) || !ctx->d_fe.ensure(n * sizeof(FastEntry)) ||
+        size_t aux_b = N * sizeof(FastAux);
+        if (!ctx->d_aux.ensure(aux_b) || !ctx->d_fe.ensure(N * sizeof(FastEntry)) ||
             !ctx->d_fb.ensure((slots + 1) * sizeof(FastBlock)) || !ctx->d_plist.ensure(3 * (slots + 1) * 4) ||
-            !ctx->d_glist.ensure(n * 4) || !ctx->d_fdesc.ensure((ndesc + 4) * 4))
+            !ctx->d_glist.ensure(N * 4) || !ctx->d_fdesc.ensure((ndesc + 4) * 4))
             return fail(ctx, ZPB_E_NOMEM, "fast-path scratch allocation failed");
         CK(ctx, cudaMemcpyAsync(ctx->d_aux.p, h_aux, aux_b, cudaMemcpyHostToDevice, s));
         const FastEntry *d_fe = (const FastEntry *)ctx->d_fe.p;
         FastBlock *d_fb = (FastBlock *)ctx->d_fb.p;
         u32 *d_plist = (u32 *)ctx->d_plist.p, *d_glist = (u32 *)ctx->d_glist.p, *d_fdesc = (u32 *)ctx->d_fdesc.p;
         CK(ctx, cudaEventRecord(ctx->evs[0], s));
-        lz4_fast_scan_kernel<<<(u32)((n + 255) / 256), 256, 0, s>>>(
-            d_archive, archive_size, d_e, d_ord, (u32)n, (const FastAux *)ctx->d_aux.p, (FastEntry *)ctx->d_fe.p,
+        if (!jobs.empty()) {
+            // the candidates' framing -> their pseudo-rows (or inert rows, and the parent as it is)
+            split_index_kernel<<<(u32)jobs.size(), 32, SPLIT_SMEM, s>>>(d_archive, (zpb_entry *)ctx->d_desc.p,
+                                                                       (FastAux *)ctx->d_aux.p, (const SplitJob *)ctx->d_jobs.p);
+            CK(ctx, cudaGetLastError());
+            ctx->launches += 1;
+        }
+        lz4_fast_scan_kernel<<<(u32)((N + 255) / 256), 256, 0, s>>>(
+            d_archive, archive_size, d_e, d_ord, (u32)N, (const FastAux *)ctx->d_aux.p, (FastEntry *)ctx->d_fe.p,
             d_fb, d_plist, (u32)(slots + 1), cnt, d_glist, (u32 *)ctx->d_zlist.p, d_status, d_digest);
         CK(ctx, cudaGetLastError());
         CK(ctx, cudaEventRecord(ctx->evs[1], s));
@@ -520,20 +595,20 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
                         const u32 *n_ptr) {
             lz4_fast_exec_kernel<<<ctx->sm_count * ctas, 32 * FAST_EXEC_WARPS, FAST_EXEC_SMEM, st>>>(
                 d_archive, archive_size, d_out, d_e, list, nl, work, d_fe, d_fb, d_fdesc, cnt, d_glist, d_status, d_digest,
-                ctx->cur_partials, defer, defer_len, n_ptr);
+                d_part, defer, defer_len, n_ptr);
             return cudaGetLastError();
         };
         const u32 *d_xord = overlap ? (const u32 *)ctx->d_order2.p : d_ord;
         const int early = overlap ? (set.early_ctas > 0 && set.early_ctas <= k2_ctas ? set.early_ctas : (k2_ctas > 1 ? k2_ctas - 1 : 1))
                                   : k2_ctas;
         u32 *d_defer = overlap ? (u32 *)ctx->d_defer.p : nullptr;
-        if (lz4_work) CK(ctx, exec(early, s, d_xord, (u32)n, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
+        if (lz4_work) CK(ctx, exec(early, s, d_xord, (u32)N, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
         if (overlap && !lz4_work) {
             CK(ctx, cudaStreamWaitEvent(s, ctx->ev_p1, 0));
         } else if (overlap) {
             if (k2_ctas > early) {
                 CK(ctx, cudaStreamWaitEvent(ctx->stream_b, ctx->ev_p1, 0));
-                CK(ctx, exec(k2_ctas - early, ctx->stream_b, d_xord, (u32)n, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
+                CK(ctx, exec(k2_ctas - early, ctx->stream_b, d_xord, (u32)N, cnt + CNT_EXEC_WORK, d_defer, cnt + CNT_DEFER, nullptr));
                 CK(ctx, cudaEventRecord(ctx->ev_xb, ctx->stream_b));
                 CK(ctx, cudaStreamWaitEvent(s, ctx->ev_xb, 0));
                 ctx->launches += 1;
@@ -561,7 +636,17 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
     }
     CK(ctx, cudaEventRecord(ctx->evs[4], s));
     if (any_zstd) {
-        CK(ctx, launch_zstd(ctx, s, d_archive, d_out, d_e, d_status, d_digest));
+        CK(ctx, launch_zstd(ctx, s, d_archive, d_out, d_e, d_status, d_digest, false, N, nullptr));
+        ctx->launches += 1;
+    }
+    if (any_frames) {
+        CK(ctx, launch_zstd(ctx, s, d_archive, d_out, d_e, d_status, d_digest, true, N, d_part));
+        ctx->launches += 1;
+    }
+    if (!jobs.empty()) {
+        xxh3_chain_batch_kernel<<<(u32)jobs.size(), 32, 0, s>>>((const SplitJob *)ctx->d_jobs.p, d_e, d_part, d_out,
+                                                                d_status, d_digest);
+        CK(ctx, cudaGetLastError());
         ctx->launches += 1;
     }
     CK(ctx, cudaEventRecord(ctx->evs[5], s));
@@ -574,9 +659,32 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         CK(ctx, cudaEventElapsedTime(&ctx->stage_ms[1], ctx->ev_p0, ctx->ev_p1));   // parse, on its own stream when overlapped
         CK(ctx, cudaEventElapsedTime(&ctx->stage_ms[2], ctx->ev_x0, ctx->ev_x1));   // execute: every grid
     }
-    if (any_zstd) CK(ctx, cudaEventElapsedTime(&ctx->zstd_ms, ctx->evs[4], ctx->evs[5]));
-    if (digest) memcpy(digest, h_res, n * sizeof(u64));
-    if (status) memcpy(status, h_res + n * sizeof(u64), n * sizeof(int));
+    if (any_zstd || any_frames) CK(ctx, cudaEventElapsedTime(&ctx->zstd_ms, ctx->evs[4], ctx->evs[5]));
+    const u64 *h_dg = (const u64 *)h_res;
+    const int *h_st = (const int *)(h_res + N * sizeof(u64));
+    // split entries whose pseudo-rows did not all decode (corrupt, or a shape only the whole-entry kernels judge): decoded
+    // again, unsplit, so that they get exactly the verdict they would have had unsplit
+    std::vector<zpb_entry> redo;
+    std::vector<u32> redo_at;
+    for (const SplitJob &j : jobs)
+        if (h_st[j.parent] == ZPB_ST_SPLIT_RETRY) { redo.push_back(entries[j.parent]); redo_at.push_back(j.parent); }
+    if (digest) memcpy(digest, h_dg, n * sizeof(u64));
+    if (status) memcpy(status, h_st, n * sizeof(int));
+    if (!redo.empty()) {
+        std::vector<int32_t> st(redo.size());
+        std::vector<u64> dg(redo.size());
+        const float first_ms = ctx->unpack_ms;
+        ctx->no_split = true;
+        const int rc = unpack_device_impl(ctx, d_archive, archive_size, d_out, out_size, redo.data(), redo.size(),
+                                          st.data(), dg.data(), s);
+        ctx->no_split = false;
+        if (rc != ZPB_OK) return rc;
+        ctx->unpack_ms += first_ms;
+        for (size_t k = 0; k < redo.size(); ++k) {
+            if (status) status[redo_at[k]] = st[k];
+            if (digest) digest[redo_at[k]] = dg[k];
+        }
+    }
     return ZPB_OK;
 }
 
