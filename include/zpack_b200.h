@@ -106,6 +106,29 @@ int zpb_unpack_device(zpb_ctx *ctx, const uint8_t *d_archive, uint64_t archive_s
                       uint8_t *d_out, uint64_t out_size, const zpb_entry *entries, uint64_t n,
                       int32_t *status, uint64_t *digest, void *stream);
 
+/* Enqueue the unpack of n entries on `stream` and return without waiting for the GPU.  entries: HOST array, fully
+ * consumed before the call returns (the caller may reuse it at once).  d_status (int32_t[n]) / d_digest (uint64_t[n]):
+ * DEVICE arrays, written in stream order — the same values zpb_unpack_device returns for the same batch.
+ *  - Argument errors (a NULL pointer, NULL d_status / d_digest with n > 0, an output slot outside out_size, a dst_off
+ *    that leaves the slot unaligned, too many entries) return before anything is enqueued.
+ *  - Output bytes, statuses and digests equal zpb_unpack_device's for every entry, large split entries included: a split
+ *    entry with a 64 KB piece that did not decode is decoded again whole on the device, by the decoder it would have
+ *    reached unsplit.
+ *  - The call waits on the host for two things only: the previous call's descriptor upload, before it reuses the
+ *    context's pinned staging, and scratch growth (a batch larger than any before on this context).  It never waits
+ *    for kernels.  d_archive, d_out and the result arrays must stay valid until the stream reaches them.
+ *  - Calls on one context run in call order, whatever stream each is given: a call's work starts after the previous
+ *    call's has ended.  Every synchronous call on the context that uses its scratch (zpb_unpack_device, zpb_unpack_host,
+ *    zpb_pack_*, zpb_xxh3_*, the block and container calls) first waits for the queued calls.
+ *  - zpb_last_kernel_ms, zpb_last_stage_ms and zpb_last_zstd_ms describe the last call; after this one they wait for
+ *    its kernels before they answer.
+ *  - A device error that appears after the call has returned is reported by the next call or getter on the context that
+ *    waits for the queued work.
+ *  - Not capture-safe: scratch may be allocated during a call. */
+int zpb_unpack_device_async(zpb_ctx *ctx, const uint8_t *d_archive, uint64_t archive_size, uint8_t *d_out,
+                            uint64_t out_size, const zpb_entry *entries, uint64_t n, int32_t *d_status,
+                            uint64_t *d_digest, void *stream);
+
 /* Same with host buffers: copies [lo,hi) of the archive that the entries touch to the device,
  * unpacks, copies each entry's uncomp_size bytes back into h_out + dst_off.  Batches of more than a few
  * hundred MB are pipelined in chunks over several streams (H2D, kernels and D2H of different chunks

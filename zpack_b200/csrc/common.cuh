@@ -41,6 +41,10 @@ enum CounterSlot : u32 {
     CNT_ZSTD_FRAMES_WORK = 16, // work counter of zstd_unpack_kernel over the frame list
     CNT_LIGHT_FIRST = 17,      // light-list length the first parse launch walked (the last launch walks the rest)
     CNT_PARSE_LAST_WORK = 18,  // work counter of the last parse launch
+    CNT_RETRY_LZ4 = 19,        // zpb_unpack_device_async: length of the list of split LZ4 parents decoded again whole,
+    CNT_RETRY_LZ4_WORK = 20,   // and the general kernel's work counter over it
+    CNT_RETRY_ZSTD = 21,       // the same for split zstd parents and zstd_unpack_kernel<ZsHasher>
+    CNT_RETRY_ZSTD_WORK = 22,
     CNT_PACK_BLOCKS_WORK = 32, // work counter of lz4_pack_blocks_kernel
     CNT_HC_MATCH_WORK = 48,    // work counter of lz4hc_match_kernel
     CNT_SLOTS = 64             // size of the block in u32 words

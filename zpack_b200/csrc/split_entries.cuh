@@ -82,15 +82,17 @@ ZPB_HD u32 split_zstd_block(u32 bh, u64 left) {
     return type == 3 || csz > left ? ~0u : csz;
 }
 
-// Internal status of a split parent whose pseudo-rows did not all decode: the host decodes it again, unsplit.
+// Internal status of a split parent whose pseudo-rows did not all decode: it is decoded again, unsplit (by the host in
+// zpb_unpack_device, after split_retry_kernel in zpb_unpack_device_async).
 #define ZPB_ST_SPLIT_RETRY 0x5350u
 
-struct SplitJob {      // host -> pre-pass -> chain kernel, one per candidate
+struct SplitJob {      // host -> pre-pass -> chain kernel -> retry kernel, one per candidate
     u64 kib0;          // its first KiB in the batch's stripe-sum array
     u64 desc_base;     // LZ4: descriptor words reserved for its blocks (fast_scan_lz4's layout)
     u32 parent;        // the caller's row
     u32 row0, nrows;   // its pseudo-rows: [row0, row0 + nrows), nrows = ceil(uncomp_size / 64 KB)
     u32 slot_base;     // LZ4: its FastBlock slots
+    u32 method;        // the parent's method (ZPB_METHOD_LZ4 / _ZSTD), which the pre-pass replaces with ZPB_M_SPLIT
 };
 
 #define SPLIT_CHUNK 65536u                       // entry bytes per stage; a header starting in a stage is walked there
@@ -214,12 +216,29 @@ split_index_kernel(const u8 *__restrict__ archive, zpb_entry *entries, FastAux *
     }
 }
 
+// One thread per candidate, after xxh3_chain_batch_kernel (zpb_unpack_device_async): a parent marked ZPB_ST_SPLIT_RETRY
+// gets its method back and joins the list of the whole-entry decoder it would have reached unsplit, so that its status
+// is that path's.  LZ4 -> lz4_list, for the general kernel, which judges every LZ4 entry the fast path declines (a
+// fast-path decode of a valid frame and the general kernel's agree); zstd -> zstd_list, for zstd_unpack_kernel<ZsHasher>.
+// The lists' lengths are counted at CNT_RETRY_LZ4 and CNT_RETRY_ZSTD.
+__global__ void __launch_bounds__(128)
+split_retry_kernel(const SplitJob *__restrict__ jobs, u32 njobs, zpb_entry *entries, const int *__restrict__ status,
+                   u32 *lz4_list, u32 *zstd_list, u32 *counters) {
+    const u32 t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= njobs) return;
+    const SplitJob j = jobs[t];
+    if (status[j.parent] != (int)ZPB_ST_SPLIT_RETRY) return;
+    entries[j.parent].method = j.method;
+    if (j.method == ZPB_METHOD_ZSTD) zstd_list[atomicAdd(&counters[CNT_RETRY_ZSTD], 1u)] = j.parent;
+    else lz4_list[atomicAdd(&counters[CNT_RETRY_LZ4], 1u)] = j.parent;
+}
+
 #ifndef ZPB_SIM   // the chain's inline PTX has no CPU emulation
 #include "xxh3_chain.cuh"
 
 // One warp per candidate, after every pseudo-row has decoded: the XXH3 chain over the entry's stripe sums, the tail and
 // the merge (xxh3_chain_body), then the parent's status and digest as the one-warp path reports them.  A parent with a
-// pseudo-row that did not decode is marked ZPB_ST_SPLIT_RETRY for the host's unsplit pass.
+// pseudo-row that did not decode is marked ZPB_ST_SPLIT_RETRY for the unsplit pass.
 __global__ void __launch_bounds__(32)
 xxh3_chain_batch_kernel(const SplitJob *__restrict__ jobs, const zpb_entry *__restrict__ entries, const u64 *partials,
                         const u8 *out, int *status, u64 *digest) {

@@ -161,10 +161,19 @@ struct zpb_ctx {
     // large entries of a batch decoded block-parallel (split_entries.cuh): candidates, their stripe sums
     std::vector<SplitJob> h_jobs;
     DevBuf d_jobs, d_bpart;
+    DevBuf d_rlist;                    // zpb_unpack_device_async: the split parents decoded again whole, LZ4 then zstd
     bool no_split = false;             // set during the unsplit pass over the entries whose pseudo-rows did not all decode
     // device-resident container operations (archive_api.inl): entry table, record offsets, chunk table, totals, names; CDR walk tables
     DevBuf d_arc_e, d_arc_rec, d_arc_chunk, d_arc_work, d_arc_scan, d_arc_tot, d_arc_names, d_cdr_jump, d_cdr_cnt, d_cdr_j2, d_cdr_anchor;
     float arc_ms[3] = {0, 0, 0};       // layout + directory kernels, copy kernel, open kernels of the last call
+    // zpb_unpack_device_async: the end of the last queued call (every unpack call's stream waits for it, every synchronous
+    // call that uses the scratch above waits for it on the host), the end of the last call's uploads from h_stage, and
+    // whether the unpack timings still have to be read from evs[] (with the two flags of that call)
+    Event ev_done, ev_staged;
+    bool timing_pending = false, timed_fast = false, timed_zstd = false;
+
+    // Unpack scratch grows (and frees the old buffer) only once the queued calls that may still read it have finished.
+    bool grow(DevBuf &b, size_t n) { return n <= b.cap || (cudaEventSynchronize(ev_done) == cudaSuccess && b.ensure(n)); }
 };
 
 #define CK(ctx, call)                                                                      \
@@ -181,6 +190,29 @@ static int fail(zpb_ctx *ctx, int code, const char *msg) {
     if (ctx) ctx->err = msg;
     g_last_error = msg;
     return code;
+}
+
+// Every synchronous call that uses the context's streams or scratch starts here: its device, then the end of the queued
+// zpb_unpack_device_async calls, which share them.  A device error of a queued call is reported here.
+static cudaError_t enter(zpb_ctx *ctx) {
+    const cudaError_t e = cudaSetDevice(ctx->device);
+    return e != cudaSuccess ? e : cudaEventSynchronize(ctx->ev_done);
+}
+
+// The last unpack call's device times, from its events: at once after a synchronous call, on the first getter after
+// an asynchronous one (which waits for the events).
+static cudaError_t read_unpack_timing(zpb_ctx *ctx) {
+    if (!ctx->timing_pending) return cudaSuccess;
+    ctx->timing_pending = false;
+    cudaError_t e = cudaEventSynchronize(ctx->evs[5]);
+    if (e == cudaSuccess) e = cudaEventElapsedTime(&ctx->unpack_ms, ctx->evs[0], ctx->evs[5]);
+    if (ctx->timed_fast) {
+        for (int k = 0; k < 4 && e == cudaSuccess; ++k) e = cudaEventElapsedTime(&ctx->stage_ms[k], ctx->evs[k], ctx->evs[k + 1]);
+        if (e == cudaSuccess) e = cudaEventElapsedTime(&ctx->stage_ms[1], ctx->ev_p0, ctx->ev_p1);   // parse, on its own stream when overlapped
+        if (e == cudaSuccess) e = cudaEventElapsedTime(&ctx->stage_ms[2], ctx->ev_x0, ctx->ev_x1);   // execute: every grid
+    }
+    if (e == cudaSuccess && ctx->timed_zstd) e = cudaEventElapsedTime(&ctx->zstd_ms, ctx->evs[4], ctx->evs[5]);
+    return e;
 }
 
 extern "C" int zpb_abi_version(void) { return ZPB_ABI_VERSION; }
@@ -223,7 +255,9 @@ extern "C" zpb_ctx *zpb_create(int device) {
         cudaEventCreateWithFlags(&ctx->ev_scan.h, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&ctx->ev_xb.h, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreate(&ctx->ev_p0.h) != cudaSuccess || cudaEventCreate(&ctx->ev_p1.h) != cudaSuccess ||
-        cudaEventCreate(&ctx->ev_x0.h) != cudaSuccess || cudaEventCreate(&ctx->ev_x1.h) != cudaSuccess) {
+        cudaEventCreate(&ctx->ev_x0.h) != cudaSuccess || cudaEventCreate(&ctx->ev_x1.h) != cudaSuccess ||
+        cudaEventCreateWithFlags(&ctx->ev_done.h, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&ctx->ev_staged.h, cudaEventDisableTiming) != cudaSuccess) {
         g_last_error = "second stream setup failed"; return nullptr;
     }
     if (cudaFuncSetAttribute(lz4_fast_parse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -270,6 +304,7 @@ extern "C" zpb_ctx *zpb_create(int device) {
 extern "C" void zpb_destroy(zpb_ctx *ctx) {
     if (!ctx) return;
     cudaSetDevice(ctx->device);
+    cudaEventSynchronize(ctx->ev_done);   // queued calls still read the scratch
     ctx->workers.clear();
     delete ctx;   // its scratch, streams and events release themselves
 }
@@ -297,12 +332,14 @@ extern "C" int zpb_set_tuning(zpb_ctx *ctx, int group_lanes, int ctas_per_sm) {
 
 extern "C" int zpb_last_stage_ms(const zpb_ctx *ctx, float *ms4) {
     if (!ctx || !ms4) return ZPB_E_ARG;
+    CK(const_cast<zpb_ctx *>(ctx), read_unpack_timing(const_cast<zpb_ctx *>(ctx)));
     for (int k = 0; k < 4; ++k) ms4[k] = ctx->stage_ms[k];
     return ZPB_OK;
 }
 
 extern "C" int zpb_last_zstd_ms(const zpb_ctx *ctx, float *ms) {
     if (!ctx || !ms) return ZPB_E_ARG;
+    CK(const_cast<zpb_ctx *>(ctx), read_unpack_timing(const_cast<zpb_ctx *>(ctx)));
     *ms = ctx->zstd_ms;
     return ZPB_OK;
 }
@@ -321,6 +358,7 @@ extern "C" int zpb_debug_zstd_profile(unsigned long long *out8) {
 // unsplit kernel), CNT_SPLIT_RETRIES and CNT_GENERAL (entries handed to the general decoder)
 extern "C" int zpb_debug_counters(zpb_ctx *ctx, unsigned *out16) {
     if (!ctx || !out16 || !ctx->d_counter.p) return ZPB_E_ARG;
+    CK(ctx, enter(ctx));
     return cudaMemcpy(out16, ctx->d_counter.p, 16 * sizeof(u32), cudaMemcpyDeviceToHost) == cudaSuccess ? ZPB_OK : ZPB_E_CUDA;
 }
 
@@ -338,6 +376,7 @@ extern "C" int zpb_set_fast_path(zpb_ctx *ctx, int enabled) {
 
 extern "C" int zpb_last_kernel_ms(const zpb_ctx *ctx, float *unpack_ms, float *pack_ms) {
     if (!ctx) return ZPB_E_ARG;
+    CK(const_cast<zpb_ctx *>(ctx), read_unpack_timing(const_cast<zpb_ctx *>(ctx)));
     if (unpack_ms) *unpack_ms = ctx->unpack_ms;
     if (pack_ms) *pack_ms = ctx->pack_ms;
     return ZPB_OK;
@@ -394,10 +433,13 @@ static bool split_candidate(const zpb_entry &e, u64 archive_size) {
            e.comp_size <= archive_size - e.src_off;
 }
 
-static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_size, u8 *d_out,
-                              u64 out_size, const zpb_entry *entries, u64 n, int32_t *status,
-                              u64 *digest, cudaStream_t s) {
-    if (n == 0) return ZPB_OK;
+// Enqueues the unpack of entries[0, n) (n > 0) on s, after the context's previous call, and returns without waiting for
+// the kernels.  Argument errors return before anything is enqueued.  The batch's *rows rows (the caller's n, then the
+// split entries' pseudo-rows) leave their digests at d_res[0, rows) and their statuses after them; evs[5] marks the end.
+// device_retry: split parents marked ZPB_ST_SPLIT_RETRY are decoded again whole on the device (split_retry_kernel);
+// otherwise they keep that mark for the caller's unsplit pass.
+static int unpack_enqueue(zpb_ctx *ctx, const u8 *d_archive, u64 archive_size, u8 *d_out, u64 out_size,
+                          const zpb_entry *entries, u64 n, cudaStream_t s, bool device_retry, u64 *rows) {
     if (n > 0x7fffffffull) return fail(ctx, ZPB_E_ARG, "too many entries in one batch");
     const bool internal = ctx->cur_partials != nullptr;   // method codes above a byte are internal (comp_method is a u8, lib/zpack.h:79)
     // Large entries (split_entries.cuh): one job per candidate, its pseudo-rows after the caller's n rows.  The rows stay
@@ -414,6 +456,7 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
                 j.nrows = (u32)((entries[i].uncomp_size + 65535) >> 16);
                 j.kib0 = kibs;
                 j.desc_base = 0; j.slot_base = 0;
+                j.method = entries[i].method;
                 N += j.nrows;
                 kibs += (entries[i].uncomp_size + 1023) >> 10;
                 jobs.push_back(j);
@@ -421,9 +464,14 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
     if (N > 0x7fffffffull) return fail(ctx, ZPB_E_ARG, "too many entries in one batch");
     size_t desc_b = N * sizeof(zpb_entry), ord_b = N * sizeof(u32);
     size_t res_b = N * (sizeof(int) + sizeof(u64));
-    if (!ctx->d_desc.ensure(desc_b) || !ctx->d_order.ensure(ord_b) || !ctx->d_res.ensure(res_b + 64) ||
-        !ctx->d_counter.ensure(CNT_SLOTS * sizeof(u32)) || !ctx->d_order2.ensure(ord_b) || !ctx->d_defer.ensure(ord_b) ||
-        !ctx->h_stage.ensure(desc_b + 2 * ord_b + res_b + 64 + N * sizeof(FastAux)))
+    // staging: descriptors, order, results (zpb_unpack_device), fast-path layout, execute order, jobs
+    const size_t jobs_at = (desc_b + 2 * ord_b + res_b + 64 + N * sizeof(FastAux) + 15) & ~(size_t)15;
+    const size_t jobs_b = jobs.size() * sizeof(SplitJob);
+    // the staging may still feed the uploads of a queued call
+    CK(ctx, cudaEventSynchronize(ctx->ev_staged));
+    if (!ctx->grow(ctx->d_desc, desc_b) || !ctx->grow(ctx->d_order, ord_b) || !ctx->grow(ctx->d_res, res_b + 64) ||
+        !ctx->grow(ctx->d_counter, CNT_SLOTS * sizeof(u32)) || !ctx->grow(ctx->d_order2, ord_b) ||
+        !ctx->grow(ctx->d_defer, ord_b) || !ctx->h_stage.ensure(jobs_at + jobs_b))
         return fail(ctx, ZPB_E_NOMEM, "scratch allocation failed");
 
     // ---- one pass over the descriptors (the GPU idles while the host prepares a batch, so this is kept to a single
@@ -496,35 +544,45 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         for (u64 k = ncheap; k < N; ++k) h_order2[k] = h_order[k - ncheap];
     }
 
-    if ((any_zstd || any_frames) && (!ctx->d_zlist.ensure(N * 8) ||
-                     !ctx->d_zlit.ensure((size_t)std::max(ctx->zs_grid, ctx->zs_grid_part) * ZS_WARPS * ZS_LIT_SCRATCH)))
+    if ((any_zstd || any_frames) && (!ctx->grow(ctx->d_zlist, N * 8) ||
+                     !ctx->grow(ctx->d_zlit, (size_t)std::max(ctx->zs_grid, ctx->zs_grid_part) * ZS_WARPS * ZS_LIT_SCRATCH)))
         return fail(ctx, ZPB_E_NOMEM, "zstd scratch allocation failed");
+    if (!jobs.empty() && (!ctx->grow(ctx->d_jobs, jobs_b) || !ctx->grow(ctx->d_bpart, (kibs + 1) * 64) ||
+                          (device_retry && !ctx->grow(ctx->d_rlist, 2 * jobs.size() * sizeof(u32)))))
+        return fail(ctx, ZPB_E_NOMEM, "split scratch allocation failed");
+    const Settings &set = ctx->set;
+    const size_t aux_b = N * sizeof(FastAux);
+    if (set.fast && (!ctx->grow(ctx->d_aux, aux_b) || !ctx->grow(ctx->d_fe, N * sizeof(FastEntry)) ||
+                     !ctx->grow(ctx->d_fb, (slots + 1) * sizeof(FastBlock)) || !ctx->grow(ctx->d_plist, 3 * (slots + 1) * 4) ||
+                     !ctx->grow(ctx->d_glist, N * 4) || !ctx->grow(ctx->d_fdesc, (ndesc + 4) * 4)))
+        return fail(ctx, ZPB_E_NOMEM, "fast-path scratch allocation failed");
     ctx->zstd_ms = 0.f;
     u64 *d_digest = (u64 *)ctx->d_res.p;
     int *d_status = (int *)((u8 *)ctx->d_res.p + N * sizeof(u64));
     const zpb_entry *d_e = (const zpb_entry *)ctx->d_desc.p;
     const u32 *d_ord = (const u32 *)ctx->d_order.p;
     u32 *cnt = (u32 *)ctx->d_counter.p;   // slots: CounterSlot (common.cuh)
-    u64 *d_part = ctx->cur_partials;      // stripe sums of 64 KB rows: the shard's, or the batch's split entries'
-    if (!jobs.empty()) {
-        if (!ctx->d_jobs.ensure(jobs.size() * sizeof(SplitJob)) || !ctx->d_bpart.ensure((kibs + 1) * 64))
-            return fail(ctx, ZPB_E_NOMEM, "split scratch allocation failed");
-        d_part = (u64 *)ctx->d_bpart.p;
-        CK(ctx, cudaMemcpyAsync(ctx->d_jobs.p, jobs.data(), jobs.size() * sizeof(SplitJob), cudaMemcpyHostToDevice, s));
-    }
+    u64 *d_part = jobs.empty() ? ctx->cur_partials : (u64 *)ctx->d_bpart.p;   // stripe sums of 64 KB rows: the shard's, or the batch's split entries'
+    const bool overlap = set.overlap != 0;
 
+    // ---- uploads, after the context's previous call, all from the staging (a pageable source could make the copy wait
+    // for the stream)
+    CK(ctx, cudaStreamWaitEvent(s, ctx->ev_done, 0));
+    if (!jobs.empty()) {
+        memcpy(hs + jobs_at, jobs.data(), jobs_b);
+        CK(ctx, cudaMemcpyAsync(ctx->d_jobs.p, hs + jobs_at, jobs_b, cudaMemcpyHostToDevice, s));
+    }
     CK(ctx, cudaMemcpyAsync(ctx->d_desc.p, h_desc, desc_b, cudaMemcpyHostToDevice, s));
     CK(ctx, cudaMemcpyAsync(ctx->d_order.p, h_order, ord_b, cudaMemcpyHostToDevice, s));
     CK(ctx, cudaMemsetAsync(ctx->d_counter.p, 0, CNT_SLOTS * sizeof(u32), s));
-    const Settings &set = ctx->set;
+    if (set.fast) {
+        CK(ctx, cudaMemcpyAsync(ctx->d_aux.p, h_aux, aux_b, cudaMemcpyHostToDevice, s));
+        if (overlap) CK(ctx, cudaMemcpyAsync(ctx->d_order2.p, h_order2, ord_b, cudaMemcpyHostToDevice, s));
+    }
+    CK(ctx, cudaEventRecord(ctx->ev_staged, s));
+
     if (set.fast) {
         // ---- scan -> parse -> exec (lz4_fast.cuh), then the general kernel over whatever they declined
-        size_t aux_b = N * sizeof(FastAux);
-        if (!ctx->d_aux.ensure(aux_b) || !ctx->d_fe.ensure(N * sizeof(FastEntry)) ||
-            !ctx->d_fb.ensure((slots + 1) * sizeof(FastBlock)) || !ctx->d_plist.ensure(3 * (slots + 1) * 4) ||
-            !ctx->d_glist.ensure(N * 4) || !ctx->d_fdesc.ensure((ndesc + 4) * 4))
-            return fail(ctx, ZPB_E_NOMEM, "fast-path scratch allocation failed");
-        CK(ctx, cudaMemcpyAsync(ctx->d_aux.p, h_aux, aux_b, cudaMemcpyHostToDevice, s));
         const FastEntry *d_fe = (const FastEntry *)ctx->d_fe.p;
         FastBlock *d_fb = (FastBlock *)ctx->d_fb.p;
         u32 *d_plist = (u32 *)ctx->d_plist.p, *d_glist = (u32 *)ctx->d_glist.p, *d_fdesc = (u32 *)ctx->d_fdesc.p;
@@ -546,12 +604,10 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         // three launches sharing the work counters: two CTAs per SM at once (they fill the SMs as parse CTAs retire and
         // never wait: an entry whose blocks are not parsed yet is put aside), the third CTA per SM once the parse kernel
         // has finished, and a last pass over the entries that were put aside.
-        const bool overlap = set.overlap != 0;
         const int k2_ctas = set.exec_ctas;
         const int k1_ctas = set.ctas_per_sm > 0 ? set.ctas_per_sm : 3;
         cudaStream_t sp = overlap ? ctx->stream_p : s;
         if (overlap) {
-            CK(ctx, cudaMemcpyAsync(ctx->d_order2.p, h_order2, ord_b, cudaMemcpyHostToDevice, s));
             CK(ctx, cudaEventRecord(ctx->ev_scan, s));
             CK(ctx, cudaStreamWaitEvent(sp, ctx->ev_scan, 0));
         }
@@ -649,17 +705,50 @@ static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_siz
         CK(ctx, cudaGetLastError());
         ctx->launches += 1;
     }
+    if (device_retry && !jobs.empty()) {
+        // parents whose pseudo-rows did not all decode: whole, through the decoder each would have reached unsplit
+        const u32 J = (u32)jobs.size();
+        u32 *d_rlist = (u32 *)ctx->d_rlist.p;
+        split_retry_kernel<<<(J + 127) / 128, 128, 0, s>>>((const SplitJob *)ctx->d_jobs.p, J, (zpb_entry *)ctx->d_desc.p,
+                                                          d_status, d_rlist, d_rlist + J, cnt);
+        CK(ctx, cudaGetLastError());
+        ctx->launches += 1;
+        bool any_lz4_job = false, any_zstd_job = false;
+        for (const SplitJob &j : jobs) (j.method == ZPB_METHOD_ZSTD ? any_zstd_job : any_lz4_job) = true;
+        if (any_lz4_job) {
+            CK(ctx, launch_general(ctx, s, d_archive, archive_size, d_out, d_e, d_rlist, 0u, cnt + CNT_RETRY_LZ4,
+                                   cnt + CNT_RETRY_LZ4_WORK, d_status, d_digest));
+            ctx->launches += 1;
+        }
+        if (any_zstd_job) {
+            zstd_unpack_kernel<ZsHasher><<<ctx->zs_grid, ZS_WARPS * 32, ZS_WARPS * sizeof(ZstdShared), s>>>(
+                d_archive, d_out, d_e, d_rlist + J, cnt + CNT_RETRY_ZSTD, cnt + CNT_RETRY_ZSTD_WORK, (u8 *)ctx->d_zlit.p,
+                d_status, d_digest, nullptr);
+            CK(ctx, cudaGetLastError());
+            ctx->launches += 1;
+        }
+    }
     CK(ctx, cudaEventRecord(ctx->evs[5], s));
-    u8 *h_res = hs + desc_b + ord_b;
+    ctx->timing_pending = true;
+    ctx->timed_fast = set.fast != 0;
+    ctx->timed_zstd = any_zstd || any_frames;
+    *rows = N;
+    return ZPB_OK;
+}
+
+static int unpack_device_impl(zpb_ctx *ctx, const u8 *d_archive, u64 archive_size, u8 *d_out,
+                              u64 out_size, const zpb_entry *entries, u64 n, int32_t *status,
+                              u64 *digest, cudaStream_t s) {
+    if (n == 0) return ZPB_OK;
+    u64 N = 0;
+    const int rc0 = unpack_enqueue(ctx, d_archive, archive_size, d_out, out_size, entries, n, s, false, &N);
+    if (rc0 != ZPB_OK) return rc0;
+    const size_t res_b = N * (sizeof(int) + sizeof(u64));
+    u8 *h_res = (u8 *)ctx->h_stage.p + N * (sizeof(zpb_entry) + sizeof(u32));   // after the descriptors and the order
     CK(ctx, cudaMemcpyAsync(h_res, ctx->d_res.p, res_b, cudaMemcpyDeviceToHost, s));
     CK(ctx, cudaStreamSynchronize(s));
-    CK(ctx, cudaEventElapsedTime(&ctx->unpack_ms, ctx->evs[0], ctx->evs[5]));
-    if (set.fast) {
-        for (int k = 0; k < 4; ++k) CK(ctx, cudaEventElapsedTime(&ctx->stage_ms[k], ctx->evs[k], ctx->evs[k + 1]));
-        CK(ctx, cudaEventElapsedTime(&ctx->stage_ms[1], ctx->ev_p0, ctx->ev_p1));   // parse, on its own stream when overlapped
-        CK(ctx, cudaEventElapsedTime(&ctx->stage_ms[2], ctx->ev_x0, ctx->ev_x1));   // execute: every grid
-    }
-    if (any_zstd || any_frames) CK(ctx, cudaEventElapsedTime(&ctx->zstd_ms, ctx->evs[4], ctx->evs[5]));
+    CK(ctx, read_unpack_timing(ctx));
+    const std::vector<SplitJob> &jobs = ctx->h_jobs;
     const u64 *h_dg = (const u64 *)h_res;
     const int *h_st = (const int *)(h_res + N * sizeof(u64));
     // split entries whose pseudo-rows did not all decode (corrupt, or a shape only the whole-entry kernels judge): decoded
@@ -693,9 +782,27 @@ extern "C" int zpb_unpack_device(zpb_ctx *ctx, const uint8_t *d_archive, uint64_
                                  uint64_t n, int32_t *status, uint64_t *digest, void *stream) {
     if (!ctx || (!entries && n) || (!d_archive && archive_size) || (!d_out && out_size))
         return fail(ctx, ZPB_E_ARG, "null argument");
-    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, enter(ctx));
     cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
     return unpack_device_impl(ctx, d_archive, archive_size, d_out, out_size, entries, n, status, digest, s);
+}
+
+extern "C" int zpb_unpack_device_async(zpb_ctx *ctx, const uint8_t *d_archive, uint64_t archive_size, uint8_t *d_out,
+                                       uint64_t out_size, const zpb_entry *entries, uint64_t n, int32_t *d_status,
+                                       uint64_t *d_digest, void *stream) {
+    if (!ctx || (!entries && n) || (!d_archive && archive_size) || (!d_out && out_size) || (n && (!d_status || !d_digest)))
+        return fail(ctx, ZPB_E_ARG, "null argument");
+    if (n == 0) return ZPB_OK;
+    CK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
+    u64 N = 0;
+    const int rc = unpack_enqueue(ctx, d_archive, archive_size, d_out, out_size, entries, n, s, true, &N);
+    if (rc != ZPB_OK) return rc;
+    CK(ctx, cudaMemcpyAsync(d_digest, ctx->d_res.p, n * sizeof(u64), cudaMemcpyDeviceToDevice, s));
+    CK(ctx, cudaMemcpyAsync(d_status, (const u8 *)ctx->d_res.p + N * sizeof(u64), n * sizeof(int32_t),
+                            cudaMemcpyDeviceToDevice, s));
+    CK(ctx, cudaEventRecord(ctx->ev_done, s));
+    return ZPB_OK;
 }
 
 // One chunk, one stream: H2D of the touched archive range -> kernels -> D2H of every entry's output.
@@ -703,7 +810,7 @@ static int unpack_host_chunk(zpb_ctx *ctx, const uint8_t *h_archive, uint64_t ar
                              uint8_t *h_out, uint64_t out_size, const zpb_entry *entries,
                              uint64_t n, int32_t *status, uint64_t *digest) {
     if (n == 0) return ZPB_OK;
-    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, enter(ctx));
     cudaStream_t s = ctx->stream;
     // the byte range of the archive the batch touches, and of the output it owns
     u64 lo = ~0ull, hi = 0, olo = ~0ull, ohi = 0;
@@ -843,6 +950,7 @@ extern "C" int zpb_unpack_host(zpb_ctx *ctx, const uint8_t *h_archive, uint64_t 
         return r;
     });
     ctx->unpack_ms = 0.f;
+    ctx->timing_pending = false;
     for (const auto &w : ctx->workers) ctx->unpack_ms += w->unpack_ms;
     return rc;
 }
@@ -856,7 +964,7 @@ extern "C" int zpb_xxh3_device(zpb_ctx *ctx, const uint8_t *d_data, const uint64
     if (!ctx || !offsets || !lengths || !digest) return fail(ctx, ZPB_E_ARG, "null argument");
     if (n == 0) return ZPB_OK;
     if (n > 0x7fffffffull) return fail(ctx, ZPB_E_ARG, "too many ranges");
-    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, enter(ctx));
     cudaStream_t s = stream ? (cudaStream_t)stream : ctx->stream;
     size_t b = n * sizeof(u64);
     if (!ctx->d_desc.ensure(2 * b) || !ctx->d_res.ensure(b) || !ctx->d_counter.ensure(CNT_SLOTS * sizeof(u32)) ||
@@ -880,7 +988,7 @@ extern "C" int zpb_xxh3_device(zpb_ctx *ctx, const uint8_t *d_data, const uint64
 
 extern "C" int zpb_xxh3_host(zpb_ctx *ctx, const uint8_t *h_data, uint64_t length, uint64_t *digest) {
     if (!ctx || (!h_data && length) || !digest) return fail(ctx, ZPB_E_ARG, "null argument");
-    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, enter(ctx));
     if (!ctx->d_in.ensure(length + 64)) return fail(ctx, ZPB_E_NOMEM, "device staging allocation failed");
     if (length) CK(ctx, cudaMemcpyAsync(ctx->d_in.p, h_data, length, cudaMemcpyHostToDevice, ctx->stream));
     u64 off = 0;

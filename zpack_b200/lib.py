@@ -57,7 +57,7 @@ assert Entry.itemsize == 64 and File.itemsize == 64 and Block.itemsize == 16 and
 
 EXPORTS = [
     "zpb_abi_version", "zpb_create", "zpb_destroy", "zpb_last_error", "zpb_device_info",
-    "zpb_launch_count", "zpb_unpack_device", "zpb_unpack_host", "zpb_xxh3_device", "zpb_xxh3_host",
+    "zpb_launch_count", "zpb_unpack_device", "zpb_unpack_device_async", "zpb_unpack_host", "zpb_xxh3_device", "zpb_xxh3_host",
     "zpb_pack_bound", "zpb_pack_device", "zpb_pack_host", "zpb_last_kernel_ms", "zpb_last_pack_stage_ms", "zpb_set_tuning",
     "zpb_last_stage_ms", "zpb_set_fast_path", "zpb_set_overlap", "zpb_set_lz4hc", "zpb_set_zstd_entropy", "zpb_last_zstd_ms",
     "zpb_lz4_frame_index", "zpb_zstd_frame_index", "zpb_unpack_blocks_device", "zpb_blocks_digest", "zpb_last_chain_ms",
@@ -94,6 +94,7 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.zpb_launch_count.argtypes = [vp]
     lib.zpb_set_tuning.argtypes = [vp, C.c_int, C.c_int]
     lib.zpb_unpack_device.argtypes = [vp, vp, u64, vp, u64, vp, u64, vp, vp, vp]
+    lib.zpb_unpack_device_async.argtypes = [vp, vp, u64, vp, u64, vp, u64, vp, vp, vp]
     lib.zpb_unpack_host.argtypes = [vp, vp, u64, vp, u64, vp, u64, vp, vp]
     lib.zpb_xxh3_device.argtypes = [vp, vp, vp, vp, u64, vp, vp]
     lib.zpb_xxh3_host.argtypes = [vp, vp, u64, vp]
@@ -327,6 +328,17 @@ class Context:
         self._check(self.lib.zpb_unpack_device(self.h, _ptr(d_archive), archive_size, _ptr(d_out), out_size,
                                                _ptr(entries), n, _ptr(status), _ptr(digest), stream))
         return status, digest
+
+    def unpack_device_async(self, d_archive, archive_size: int, d_out, out_size: int, entries: np.ndarray, d_status,
+                            d_digest, stream: int = 0) -> None:
+        """Enqueue unpack_device's work on `stream` (a cudaStream_t, e.g. torch.cuda.current_stream().cuda_stream) and
+        return without waiting for the GPU.  d_status (int32[n]) and d_digest (uint64[n], e.g. a torch.int64 tensor) are
+        device buffers (torch tensors or raw pointers) that receive unpack_device's results in stream order; `entries`
+        may be reused as soon as the call returns."""
+        assert entries.dtype == Entry and entries.flags.c_contiguous
+        self._check(self.lib.zpb_unpack_device_async(self.h, _ptr(d_archive), archive_size, _ptr(d_out), out_size,
+                                                     _ptr(entries), len(entries), _ptr(d_status), _ptr(d_digest),
+                                                     stream))
 
     def unpack_host(self, h_archive, archive_size: int, h_out, out_size: int, entries: np.ndarray):
         """Host buffers in, host buffers out (H2D + kernels + D2H inside the call)."""
